@@ -2,7 +2,7 @@
 """Benchmark of the SO(3) diffusion hot path (BASELINE.json metric: IGSO(3) score evals/sec &
 reverse-diffusion particle-steps/sec).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n ROWS] [--L 2000]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n ROWS] [--L 2000] [--dump-outputs DIR]
 
 Headline workload (BASELINE configs[1]): one *step* = one fused launch evaluating log-density and
 score of the IGSO(3) truncated series (exactly L = 2000 terms per evaluation, no early exit) on
@@ -15,6 +15,10 @@ reference's CPU path (`cpu_baseline`) and the reference's op sequence as stock P
 
 --impl reference times the torch-CPU port of the reference's algorithm (oracle/ref_port.py; the
 pure-Python reference cannot travel to the GPU box) on the host cores for the same metric.
+
+--dump-outputs DIR writes the results of the last timed step on rank 0 as DIR/<name>.npy (logp and score;
+--impl reference: logp and logp_grad, its gradient in the rotation matrix), a fixed seeded sample of DUMP_ROWS
+rows when there are more.  The inputs are the same on every run, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -57,6 +61,7 @@ NCU_DRAM_BYTES_PER_EVAL = (169.070080e6 + 43.798272e6) / 4194304
 MMD_LANE_INSTR_PER_PAIR = 41  # executed FP32-pipe instructions per pair of the all-pairs kernel (SASS count, DESIGN.md 4.6)
 CPU_SAMPLE_ROWS = 1 << 18     # rows of the bench's own inputs the CPU legs evaluate per call
 SAMPLER_B = 1 << 16           # batch of the q_sample / p_sample CPU and CUDA-eager legs (the reference's (1000, B) fp64 table bounds it)
+DUMP_ROWS = 1 << 21           # rows --dump-outputs writes at most: 2^21 x (4 + 12) B = 32 MiB of float32 results
 
 
 def peaks():
@@ -274,6 +279,21 @@ def accuracy_of_timed_results(R, eps, logp, score, rows=1 << 16):
                        "(omega > 1e-4) and the 3-vector (omega > 1e-2: the axis of a rotation by omega is defined to ~6e-8/omega in fp32)"}
 
 
+def dump_outputs(out_dir, arrays):
+    """Write each row-major array of `arrays` (name -> tensor, rows first) as out_dir/<name>.npy.  Above DUMP_ROWS rows
+    the same rows of every array are kept, chosen by a seeded permutation: the same rows for every run with the same --n."""
+    n = next(iter(arrays.values())).shape[0]
+    idx = None
+    if n > DUMP_ROWS:
+        idx = torch.randperm(n, generator=torch.Generator().manual_seed(SEED))[:DUMP_ROWS].sort().values
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.detach()
+        if idx is not None:
+            a = a[idx.to(a.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
+
+
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -288,8 +308,10 @@ def run_reference(args):
         P.score_via_autograd(R, eps)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        P.score_via_autograd(R, eps)
+        logp, logp_grad = P.score_via_autograd(R, eps)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logp": logp, "logp_grad": logp_grad})
     val = n * args.steps / dt
     sample = "each step = 2^18 rotations (bounded sample of the 2^24-row step), E-set law, per-row eps, reference closed-form fp64 log_prob + autograd score"
     line = {
@@ -350,7 +372,10 @@ def main():
     ap.add_argument("--no-numa-bind", action="store_true", help="multi-GPU runs: leave the ranks' CPU affinity alone (A/B of the e2e leg)")
     ap.add_argument("--e2e-chunk", type=int, default=1 << 21, help="rows per chunk of the host-buffer pipeline")
     ap.add_argument("--sweep-max-log2", type=int, default=28, help="largest size of the cfg 2 sweep (2^k rotations)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     if args.impl == "reference":
@@ -400,6 +425,8 @@ def main():
     per_gpu = evals_per_s / world
     # measured error of exactly these results (rank 0; CPU work, outside every timed region)
     accuracy = accuracy_of_timed_results(R, eps, logp, score) if (rank == 0 and not args.no_accuracy) else None
+    if rank == 0 and args.dump_outputs:   # now: the legs below reuse logp / score
+        dump_outputs(args.dump_outputs, {"logp": logp, "score": score})
 
     # ---- e2e: public host-buffer API, pinned host inputs -> host results -------------------------
     # dx.ops.HostScorePipeline is the call a user with host-resident batches makes: it overlaps the H2D copy,

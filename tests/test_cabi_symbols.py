@@ -55,7 +55,11 @@ def test_binding_covers_every_compute_symbol(lib_path):
 
 
 def test_sass_is_sm100a(lib_path):
-    out = subprocess.run(["cuobjdump", "-lelf", lib_path], capture_output=True, text=True).stdout
+    from diffusion_extensions_b200 import build
+
+    # the toolkit that built the library, which need not be on PATH
+    cuobjdump = os.path.join(os.path.dirname(build.find_nvcc()), "cuobjdump")
+    out = subprocess.run([cuobjdump, "-lelf", lib_path], capture_output=True, text=True).stdout
     assert "sm_100a" in out
 
 
