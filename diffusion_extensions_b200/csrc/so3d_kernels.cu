@@ -1015,7 +1015,7 @@ __global__ void __launch_bounds__(kT2, OpMinCtas<Op>::value) rowwise_kernel_w2(c
 }
 
 template <class Op>
-int launch_rowwise_w2(const Op& op, int64_t n, void* stream, const char* name) {
+int launch_rowwise_w2(const Op& op, int64_t n, void* stream, const char* name, int ctas_per_sm = 0) {
   if (n < 0) return fail(SO3D_EINVAL, "negative n");
   if (n == 0) return 0;
   int use_tma = 1;
@@ -1040,7 +1040,7 @@ int launch_rowwise_w2(const Op& op, int64_t n, void* stream, const char* name) {
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kT2, smem) != cudaSuccess || occ < 1) occ = 1;
     resident_dev[dev] = occ;
   }
-  int ctas_per_sm = resident_dev[dev];
+  if (ctas_per_sm <= 0 || ctas_per_sm > resident_dev[dev]) ctas_per_sm = resident_dev[dev];
   if (const char* e = getenv("SO3D_CTAS_PER_SM")) {
     const int v = atoi(e);
     if (v > 0 && v < ctas_per_sm) ctas_per_sm = v;
@@ -1389,18 +1389,26 @@ struct LogpScoreOp : LogpPre<SO3D_LOGP_PREFETCH && (kMode == kClosed || kMode ==
 #ifndef SO3D_LOGP2_OUTSTAGES
 #define SO3D_LOGP2_OUTSTAGES 1
 #endif
+// The series modes use the same op: both rows' L-term recurrences run as one packed loop (igso3_series_branch_l2, the same
+// bits as the one-row kernel).
+#ifndef SO3D_SERIES2_MINCTAS
+#define SO3D_SERIES2_MINCTAS 4  // register budget of the two-row series kernel (4 CTAs of 128 threads: <= 128 registers)
+#endif
 template <int kMode>
 struct LogpScore2Op : LogpScoreOp<kMode> {
-  static_assert(kMode == kClosed || kMode == kAuto, "two-row form: HBM-bound evaluators only");
+  static constexpr bool kSeriesMode = kMode == kSeries || kMode == kSeriesAdaptive || kMode == kSeriesPure;
+  using Pre1 = typename LogpPre<true>::Pre1;
   using Pre2 = typename LogpPre<true>::Pre2;
   static constexpr int kOutStages = SO3D_LOGP2_OUTSTAGES;
   static constexpr int kInStages = 1;
-  static constexpr int kMinCtas = SO3D_LOGP2_MINCTAS;
+  static constexpr int kMinCtas = kSeriesMode ? SO3D_SERIES2_MINCTAS : SO3D_LOGP2_MINCTAS;
   int64_t n;  // rows beyond the end of a ragged tile must not touch logp / dlogf
   __device__ void row2(int64_t i0, const Pre2 (&p)[2], const Mat3 (*a9)[2], const Vec3 (*)[2], Mat3 (*)[2], Vec3 (*o3)[2], const float*) const {
     const AxisAngleL<L2> a = axis_angle_fast_l(lanes_of(a9[0][0], a9[0][1]));
     float lf2[2], g2[2];
-    if (kMode == kAuto && SO3D_LOGP2_AUTO_VOTE) {
+    if constexpr (kSeriesMode) {
+      igso3_series_branch_l2<kMode>(a.theta, L2{p[0].eps, p[1].eps}, this->L, lf2, g2);
+    } else if (kMode == kAuto && SO3D_LOGP2_AUTO_VOTE) {
       // auto: the closed form for both rows, straight-line; the rows above eps = 1 (none in a DDPM schedule) are re-evaluated by
       // the series behind ONE warp vote instead of a divergent region per row (r05j: the per-row branch scaffolding was 10 % of
       // this kernel's issue slots).  Same bits as igso3_logf_g_t<kAuto>.
@@ -2603,17 +2611,19 @@ int so3d_scale_bwd_f32(const float* R, const float* s, int s_stride, const float
 template <int kMode>
 static int launch_logp_score(const float* R, const float* eps, int eps_stride, float* logp, float* score3, float* dlogf, int64_t n, int L,
                              void* stream) {
-#if SO3D_LOGP_PREFETCH
-  if constexpr (kMode == kClosed || kMode == kAuto) {
+  constexpr bool kSeriesMode = LogpScore2Op<kMode>::kSeriesMode;
+  if constexpr (kSeriesMode || SO3D_LOGP_PREFETCH) {
     const char* lanes_env = getenv("SO3D_LOGP_LANES");
     if (!(lanes_env && atoi(lanes_env) == 1)) {
       LogpScore2Op<kMode> op2;
       op2.in9[0] = R; op2.eps = eps; op2.eps_stride = eps_stride; op2.logp = logp; op2.dlogf = dlogf; op2.out3[0] = score3;
       op2.L = L; op2.n = n;
-      return launch_rowwise_w2(op2, n, stream, "so3d_igso3_logp_score_f32");
+      // Resident CTAs per SM of the two-row series kernel, measured on B200 at 2^24 rows (profiles/r06a_series_lanes.jsonl):
+      // series / series_pure gain with every resident CTA up to the 6 that fit (series 9.39 ms at 2, 8.66 at 6), series_adaptive
+      // (a different trip count per warp) runs fastest at 3 like the one-row kernel (7.02 ms, 7.74 at 6).
+      return launch_rowwise_w2(op2, n, stream, "so3d_igso3_logp_score_f32", kMode == kSeriesAdaptive ? 3 : 0);
     }
   }
-#endif
   LogpScoreOp<kMode> op;
   op.in9[0] = R; op.eps = eps; op.eps_stride = eps_stride; op.logp = logp; op.dlogf = dlogf; op.out3[0] = score3;
   op.L = L;

@@ -133,6 +133,7 @@ SO3D_HD L mulc(float k, L a) {
 SO3D_LANEWISE1(vabs, fabsf(v))
 SO3D_LANEWISE1(vrsqrt, rsqrt_approx(v))
 SO3D_LANEWISE1(vrcp, rcp_approx(v))
+SO3D_LANEWISE1(vex2, fast_ex2(v))
 #undef SO3D_LANEWISE1
 SO3D_HD L1 vmax(L1 a, L1 b) { return L1{fmaxf(a.x, b.x)}; }
 SO3D_HD L2 vmax(L2 a, L2 b) { return L2{fmaxf(a.x, b.x), fmaxf(a.y, b.y)}; }
@@ -358,6 +359,70 @@ SO3D_HD Vec3L<L> sphere_from_uniforms_l(L ua, L ub) {
   L sp, cp;
   sincos_draw_l(fma(bc<L>(kTwoPi), ub, bc<L>(-kPi)), &sp, &cp);
   return Vec3L<L>{mul(r, cp), mul(r, sp), z};
+}
+
+// ---- the L-term series (igso3_series_terms, source form 0) on two rows ---------------------------------------------------
+// Per term, for both rows: FMUL2, 2 MUFU.EX2 (each writes its half of the register pair), 4 FFMA2, 2 FADD2, and the table
+// factors as uniform-register operands broadcast to both halves (one LDCU.64 per two terms) -- 5 issue slots + 2 MUFU per two
+// row-terms where the one-row kernel spends 2 x 9.  The one-row kernel's `A + d` with A = ex2(x) * mh is contracted by the
+// compiler into FFMA e, mh, d; the fma below is that instruction, so every lane goes through the same operations and gives
+// the same bits.  Same block structure as igso3_series_terms: the ragged top block first, then whole blocks by block index.
+struct SeriesStateL2 {
+  L2 b, d, bp, dp, b2, bp2;
+};
+template <int kUnroll>
+SO3D_HD void igso3_series_run_l2(SeriesStateL2& st, L2 kap, L2 kapp, L2 cexp, int hi, int count) {
+#pragma unroll kUnroll
+  for (int i = 0; i < count; ++i) {
+    const int l = hi - i;
+    const L2 e = vex2(mul(bc<L2>(series_mm(l)), cexp));
+    const L2 dn = fnma(kap, st.b, fma(e, bc<L2>(series_mh(l)), st.d));
+    const L2 dpn = fnma(kap, st.bp, fnma(kapp, st.b, st.dp));
+    st.b2 = st.b;
+    st.bp2 = st.bp;
+    st.b = add(st.b, dn);
+    st.bp = add(st.bp, dpn);
+    st.d = dn;
+    st.dp = dpn;
+  }
+}
+
+// log f and d log f / dw of the series modes (igso3_series_branch<kMode>, guard form 3) for two rows; `L` is the same for both
+template <int kMode>
+SO3D_HD void igso3_series_branch_l2(L2 w, L2 eps, int L, float* logf_out, float* g_out) {
+  static_assert(kMode == kSeries || kMode == kSeriesAdaptive || kMode == kSeriesPure, "series modes only");
+  int terms = L;
+  if (kMode == kSeriesAdaptive) {
+    const int t0 = igso3_series_live_terms(eps.x, L), t1 = igso3_series_live_terms(eps.y, L);
+    terms = t0 > t1 ? t0 : t1;
+#if defined(__CUDA_ARCH__)
+    terms = __reduce_max_sync(__activemask(), terms);  // warp-uniform trip count (table operands stay uniform loads)
+#endif
+#if SO3D_SERIES_ROUNDUP
+    const int up = (terms + kSeriesBlock - 1) / kSeriesBlock * kSeriesBlock;
+    terms = up <= L ? up : L;
+#endif
+  }
+  constexpr bool kGuarded = kMode != kSeriesPure;
+  const bool guard0 = kGuarded && eps.x <= kAutoSeriesEps && w.x > kSeriesGuard * eps.x;
+  const bool guard1 = kGuarded && eps.y <= kAutoSeriesEps && w.y > kSeriesGuard * eps.y;
+  float lf_c[2] = {0.f, 0.f}, g_c[2] = {0.f, 0.f};
+  if (guard0) igso3_closed_f32_outofline(w.x, eps.x, &lf_c[0], &g_c[0]);
+  if (guard1) igso3_closed_f32_outofline(w.y, eps.y, &lf_c[1], &g_c[1]);
+  L2 kap, kapp, cexp;
+  igso3_series_lane_setup(w.x, eps.x, &kap.x, &kapp.x, &cexp.x);
+  igso3_series_lane_setup(w.y, eps.y, &kap.y, &kapp.y, &cexp.y);
+  const L2 zero = bc<L2>(0.f);
+  SeriesStateL2 st{zero, zero, zero, zero, zero, zero};
+  const int ragged = terms % kSeriesBlock;
+  if (ragged) igso3_series_run_l2<1>(st, kap, kapp, cexp, terms - 1, ragged);
+  for (int blk = terms / kSeriesBlock - 1; blk >= 0; --blk)
+    igso3_series_run_l2<kSeriesBlock>(st, kap, kapp, cexp, blk * kSeriesBlock + (kSeriesBlock - 1), kSeriesBlock);
+  const L2 F = add(st.b, st.b2), dF = add(st.bp, st.bp2);
+  logf_out[0] = guard0 ? lf_c[0] : logf(2.0f * F.x);
+  g_out[0] = guard0 ? g_c[0] : dF.x / F.x;
+  logf_out[1] = guard1 ? lf_c[1] : logf(2.0f * F.y);
+  g_out[1] = guard1 ? g_c[1] : dF.y / F.y;
 }
 
 // ---- lane <-> scalar glue ------------------------------------------------------------------------------------------------
