@@ -362,26 +362,72 @@ SO3D_HD Vec3L<L> sphere_from_uniforms_l(L ua, L ub) {
 }
 
 // ---- the L-term series (igso3_series_terms, source form 0) on two rows ---------------------------------------------------
-// Per term, for both rows: FMUL2, 2 MUFU.EX2 (each writes its half of the register pair), 4 FFMA2, 2 FADD2, and the table
-// factors as uniform-register operands broadcast to both halves (one LDCU.64 per two terms) -- 5 issue slots + 2 MUFU per two
-// row-terms where the one-row kernel spends 2 x 9.  The one-row kernel's `A + d` with A = ex2(x) * mh is contracted by the
-// compiler into FFMA e, mh, d; the fma below is that instruction, so every lane goes through the same operations and gives
-// the same bits.  Same block structure as igso3_series_terms: the ragged top block first, then whole blocks by block index.
+// Per term, for both rows: FMUL2, 2 MUFU.EX2 (each writes its half of the register pair), 3 FFMA2, 3 FADD2 (4 FFMA2 and
+// 2 FADD2 in the w form), and the table factors as uniform-register operands broadcast to both halves (one LDCU.64 per two
+// terms) -- 5 issue slots + 2 MUFU per two row-terms where the one-row kernel spends 2 x 9.  The one-row kernel's `A + d`
+// with A = ex2(x) * mh is contracted by the compiler into FFMA e, mh, d; the fma below is that instruction, so every lane
+// goes through the same operations and gives the same bits.  Same block structure as igso3_series_terms: the ragged top block first, then whole blocks by block index.
+// Source-form knobs of the packed block, as SO3D_SERIES_ORDER / SO3D_SERIES_BLOCK for the one-row loop: the same operations
+// per lane in every form, only the order ptxas's list scheduler sees them in (and with it its operand-reuse flags) changes.
+//   order 0: t = fma(e, mh, d); d = t - kap b; u = d' - b; d' = u - kap b'; b += d; b' += d'
+//   order 1: the two consumers of b (u, d), then the two of kap (d, d') back to back
+//   order 2: the derivative chain first
+//   order 3: every consumer of b together (d, b += d, u), then d'
+// Measured on B200 (profiles/r07a_series_forms.jsonl, DESIGN.md 4.1): order 0 and 1 compile to the same SASS; order 3 runs
+// `series` 2.4 % faster but series_adaptive 3.6 % and the 16 384-row batch 6 % slower; blocks 16 and 64 are slower.
+#ifndef SO3D_SERIES2_ORDER
+#define SO3D_SERIES2_ORDER 0
+#endif
+#ifndef SO3D_SERIES2_BLOCK
+#define SO3D_SERIES2_BLOCK 32
+#endif
+constexpr int kSeries2Block = SO3D_SERIES2_BLOCK;
 struct SeriesStateL2 {
   L2 b, d, bp, dp, b2, bp2;
 };
+// series_dsrc over lanes
+SO3D_HD L2 series_dsrc_l2(L2 kapp, L2 b, L2 dp) {
+#if SO3D_SERIES_DERIV
+  (void)kapp;
+  return sub(dp, b);
+#else
+  return fnma(kapp, b, dp);
+#endif
+}
 template <int kUnroll>
 SO3D_HD void igso3_series_run_l2(SeriesStateL2& st, L2 kap, L2 kapp, L2 cexp, int hi, int count) {
 #pragma unroll kUnroll
   for (int i = 0; i < count; ++i) {
     const int l = hi - i;
     const L2 e = vex2(mul(bc<L2>(series_mm(l)), cexp));
-    const L2 dn = fnma(kap, st.b, fma(e, bc<L2>(series_mh(l)), st.d));
-    const L2 dpn = fnma(kap, st.bp, fnma(kapp, st.b, st.dp));
+    const L2 mh = bc<L2>(series_mh(l));
     st.b2 = st.b;
     st.bp2 = st.bp;
+#if SO3D_SERIES2_ORDER == 0
+    const L2 dn = fnma(kap, st.b, fma(e, mh, st.d));
+    const L2 dpn = fnma(kap, st.bp, series_dsrc_l2(kapp, st.b, st.dp));
     st.b = add(st.b, dn);
     st.bp = add(st.bp, dpn);
+#elif SO3D_SERIES2_ORDER == 1
+    const L2 t = fma(e, mh, st.d);
+    const L2 u = series_dsrc_l2(kapp, st.b, st.dp);
+    const L2 dn = fnma(kap, st.b, t);
+    const L2 dpn = fnma(kap, st.bp, u);
+    st.b = add(st.b, dn);
+    st.bp = add(st.bp, dpn);
+#elif SO3D_SERIES2_ORDER == 2
+    const L2 dpn = fnma(kap, st.bp, series_dsrc_l2(kapp, st.b, st.dp));
+    const L2 dn = fnma(kap, st.b, fma(e, mh, st.d));
+    st.bp = add(st.bp, dpn);
+    st.b = add(st.b, dn);
+#else
+    const L2 dn = fnma(kap, st.b, fma(e, mh, st.d));
+    const L2 bn = add(st.b, dn);
+    const L2 u = series_dsrc_l2(kapp, st.b, st.dp);
+    const L2 dpn = fnma(kap, st.bp, u);
+    st.b = bn;
+    st.bp = add(st.bp, dpn);
+#endif
     st.d = dn;
     st.dp = dpn;
   }
@@ -399,7 +445,7 @@ SO3D_HD void igso3_series_branch_l2(L2 w, L2 eps, int L, float* logf_out, float*
     terms = __reduce_max_sync(__activemask(), terms);  // warp-uniform trip count (table operands stay uniform loads)
 #endif
 #if SO3D_SERIES_ROUNDUP
-    const int up = (terms + kSeriesBlock - 1) / kSeriesBlock * kSeriesBlock;
+    const int up = (terms + kSeries2Block - 1) / kSeries2Block * kSeries2Block;
     terms = up <= L ? up : L;
 #endif
   }
@@ -414,11 +460,16 @@ SO3D_HD void igso3_series_branch_l2(L2 w, L2 eps, int L, float* logf_out, float*
   igso3_series_lane_setup(w.y, eps.y, &kap.y, &kapp.y, &cexp.y);
   const L2 zero = bc<L2>(0.f);
   SeriesStateL2 st{zero, zero, zero, zero, zero, zero};
-  const int ragged = terms % kSeriesBlock;
+  const int ragged = terms % kSeries2Block;
   if (ragged) igso3_series_run_l2<1>(st, kap, kapp, cexp, terms - 1, ragged);
-  for (int blk = terms / kSeriesBlock - 1; blk >= 0; --blk)
-    igso3_series_run_l2<kSeriesBlock>(st, kap, kapp, cexp, blk * kSeriesBlock + (kSeriesBlock - 1), kSeriesBlock);
-  const L2 F = add(st.b, st.b2), dF = add(st.bp, st.bp2);
+  for (int blk = terms / kSeries2Block - 1; blk >= 0; --blk)
+    igso3_series_run_l2<kSeries2Block>(st, kap, kapp, cexp, blk * kSeries2Block + (kSeries2Block - 1), kSeries2Block);
+  const L2 F = add(st.b, st.b2);
+#if SO3D_SERIES_DERIV
+  const L2 dF = mul(kapp, add(st.bp, st.bp2));  // series_dF
+#else
+  const L2 dF = add(st.bp, st.bp2);
+#endif
   logf_out[0] = guard0 ? lf_c[0] : logf(2.0f * F.x);
   g_out[0] = guard0 ? g_c[0] : dF.x / F.x;
   logf_out[1] = guard1 ? lf_c[1] : logf(2.0f * F.y);

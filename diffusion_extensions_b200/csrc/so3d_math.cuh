@@ -739,16 +739,18 @@ SO3D_HD void igso3_closed_f32(float w, float eps, float* logf_out, float* g_out)
 // summed by Clenshaw's backward recurrence in Reinsch's difference form.  chi_l obeys
 // chi_{l+1} = (2 - kappa) chi_l - chi_{l-1}, kappa = 4 sin^2(w/2), chi_0 = 1, chi_{-1} = -1, so with
 //     d_l = A_l - kappa b_{l+1} + d_{l+1},        b_l = b_{l+1} + d_l          (b_L = d_L = 0)
-// the sum is F = b_0 + b_1, and differentiating the recurrence w.r.t. w (kappa' = 2 sin w) gives
-//     d'_l = -kappa' b_{l+1} - kappa b'_{l+1} + d'_{l+1},   b'_l = b'_{l+1} + d'_l,   F' = b'_0 + b'_1,
-// hence d log f / dw = F'/F with no cancellation against cot(w/2) and nothing to special-case at w = 0.
+// the sum is F = b_0 + b_1.  F depends on w only through kappa, so the recurrence is differentiated w.r.t. kappa:
+//     d'_l = -b_{l+1} - kappa b'_{l+1} + d'_{l+1},   b'_l = b'_{l+1} + d'_l,   dF/dw = kappa' (b'_0 + b'_1),  kappa' = 2 sin w,
+// hence d log f / dw = F'/F with no cancellation against cot(w/2) and nothing to special-case at w = 0 (kappa' = 0 there).
+// (Differentiating w.r.t. w instead, d'_l = -kappa' b_{l+1} - kappa b'_{l+1} + d'_{l+1}, costs an fma where the kappa form
+// has a subtraction: one more register operand per term.  SO3D_SERIES_DERIV=0 keeps that form.)
 // No sin/cos of (l w) is ever formed: the previous design rotated (sin, cos)(m w) term by term and
 // re-anchored it with an exact-product sincos every 32 terms (13 FP32 + 1 MUFU per term); this form
 // needs 8 FP32 + 1 MUFU.EX2 per term, no anchors, and is MORE accurate (measured on the E-set,
 // oracle/proto_series_fp32.py: max rel err of f 1.5e-6 vs 3.4e-6 for w <= 3.5 eps; the plain
 // Clenshaw form with K = 2 cos w is 3e-4 there because of the rounding of K, hence Reinsch).
 // Per term, all fp32:  x = mm * cexp;  A = ex2(x) * mh;  t = A + d;  d = fma(-kappa, b, t);
-//   u = fma(-kappa', b, d');  d' = fma(-kappa, b', u);  b += d;  b' += d'.
+//   u = d' - b;  d' = fma(-kappa, b', u);  b += d;  b' += d'.
 // m(m+1) is exact in fp32 for m < 2896.
 //
 // The row-invariant factors {m + 1/2, m(m+1)} come from a constant-memory table and reach the FP32 pipe
@@ -757,6 +759,8 @@ SO3D_HD void igso3_closed_f32(float w, float eps, float* logf_out, float* g_out)
 // forms 117, 1-register forms 129 lanes/clk/SM -- so each factor kept out of the vector register file
 // is a direct saving.  Packing two rows per thread as f32x2 (igso3_series_branch_l2 in so3d_lanes.cuh) reads about as
 // many operand words per flop, but cuts the issue slots per row-term from 9 to 5, and issue was the binding floor: measured 10.42 -> 8.66 ms at L = 2000, 2^24 rows, the same bits (profiles/r06a_series_lanes.jsonl).
+// The kappa-form derivative then takes the packed term from 34 to 32 register words (profiles/sass_series_reads.py), with XU
+// and operand reads both at 16 clk per packed term: measured 8.65 -> 8.36 ms on B200 (profiles/r07a_series_forms.jsonl).
 // Also measured (profiles/r01l_series_ab.jsonl): deriving every second weight by a multiply, e_{l-1} = e_l rho_l,
 // rho_{l-2} = rho_l 2^(4c) (half the MUFU, +0.5 FMUL per term) is SLOWER, 12.9 vs 12.2 clk per warp-term: the
 // FP32 operand bandwidth is the wall, not the XU pipe.
@@ -775,6 +779,11 @@ SO3D_HD void igso3_closed_f32(float w, float eps, float* logf_out, float* g_out)
 #endif
 #ifndef SO3D_SERIES_ROUNDUP
 #define SO3D_SERIES_ROUNDUP 1
+#endif
+// Variable the derivative chain differentiates in: 1 (shipped) kappa, F' = kappa' (b'_0 + b'_1) after the loop; 0 w, the
+// form before it (kappa' inside the loop, one more register operand per term).  The warp-split form below stays in w.
+#ifndef SO3D_SERIES_DERIV
+#define SO3D_SERIES_DERIV 1
 #endif
 constexpr int kSeriesBlock = SO3D_SERIES_BLOCK;       // unrolled terms per block
 constexpr int kSeriesMaxTerms = 2896;  // m(m+1) is exact in fp32 below this
@@ -867,6 +876,26 @@ struct SeriesState {
   float b2, bp2; // b_{l+2}, b'_{l+2}
 };
 
+// The derivative chain's source term, the derivative of -kappa b_{l+1}: -b_{l+1} in the kappa form (a subtraction),
+// -kappa' b_{l+1} in the w form (an fma with kappa' = 2 sin w)
+SO3D_HD float series_dsrc(float kapp, float b, float dp) {
+#if SO3D_SERIES_DERIV
+  (void)kapp;
+  return dp - b;
+#else
+  return fmaf(-kapp, b, dp);
+#endif
+}
+// dF/dw from the chain's b'_0 + b'_1: times kappa' = dkappa/dw in the kappa form
+SO3D_HD float series_dF(float kapp, float bp_sum) {
+#if SO3D_SERIES_DERIV
+  return kapp * bp_sum;
+#else
+  (void)kapp;
+  return bp_sum;
+#endif
+}
+
 // terms l = hi, hi-1, ..., hi-count+1 (descending)
 template <int kUnroll>
 SO3D_HD void igso3_series_run(SeriesState& st, float kap, float kapp, float cexp, int hi, int count) {
@@ -876,7 +905,7 @@ SO3D_HD void igso3_series_run(SeriesState& st, float kap, float kapp, float cexp
 #if SO3D_SERIES_ORDER == 0
     const float A = fast_ex2(series_mm(l) * cexp) * series_mh(l);
     const float dn = fmaf(-kap, st.b, A + st.d);
-    const float dpn = fmaf(-kap, st.bp, fmaf(-kapp, st.b, st.dp));
+    const float dpn = fmaf(-kap, st.bp, series_dsrc(kapp, st.b, st.dp));
     st.b2 = st.b;
     st.bp2 = st.bp;
     st.b += dn;
@@ -884,7 +913,7 @@ SO3D_HD void igso3_series_run(SeriesState& st, float kap, float kapp, float cexp
     st.d = dn;
     st.dp = dpn;
 #elif SO3D_SERIES_ORDER == 1  // derivative chain first
-    const float dpn = fmaf(-kap, st.bp, fmaf(-kapp, st.b, st.dp));
+    const float dpn = fmaf(-kap, st.bp, series_dsrc(kapp, st.b, st.dp));
     const float A = fast_ex2(series_mm(l) * cexp) * series_mh(l);
     const float dn = fmaf(-kap, st.b, A + st.d);
     st.b2 = st.b;
@@ -894,7 +923,7 @@ SO3D_HD void igso3_series_run(SeriesState& st, float kap, float kapp, float cexp
     st.dp = dpn;
     st.d = dn;
 #elif SO3D_SERIES_ORDER == 3  // derivative chain first, each chain's updates kept together
-    const float dpn = fmaf(-kap, st.bp, fmaf(-kapp, st.b, st.dp));
+    const float dpn = fmaf(-kap, st.bp, series_dsrc(kapp, st.b, st.dp));
     st.bp2 = st.bp;
     st.bp += dpn;
     st.dp = dpn;
@@ -905,7 +934,7 @@ SO3D_HD void igso3_series_run(SeriesState& st, float kap, float kapp, float cexp
     st.d = dn;
 #else  // kap-products grouped: t = d - kap b, u = dp - kapp b
     const float t = fmaf(-kap, st.b, st.d);
-    const float u = fmaf(-kapp, st.b, st.dp);
+    const float u = series_dsrc(kapp, st.b, st.dp);
     const float dn = fmaf(fast_ex2(series_mm(l) * cexp), series_mh(l), t);
     const float dpn = fmaf(-kap, st.bp, u);
     st.b2 = st.b;
@@ -931,7 +960,7 @@ SO3D_HD SeriesAcc igso3_series_terms(float w, float eps, int L) {
   // block index as the loop variable: table offsets are provably 128-byte aligned -> LDCU.128
   for (int blk = L / kSeriesBlock - 1; blk >= 0; --blk)
     igso3_series_run<kSeriesBlock>(st, kap, kapp, cexp, blk * kSeriesBlock + (kSeriesBlock - 1), kSeriesBlock);
-  return SeriesAcc{st.b + st.b2, st.bp + st.bp2};
+  return SeriesAcc{st.b + st.b2, series_dF(kapp, st.bp + st.bp2)};
 }
 
 // terms l = 0 .. L-1 in one rolled loop (igso3_series_run<1>): bit-identical to igso3_series_terms, tiny code
@@ -946,7 +975,7 @@ SO3D_HD SeriesAcc igso3_series_terms_rolled(float w, float eps, int L) {
   SeriesState st;
   st.b = st.d = st.bp = st.dp = st.b2 = st.bp2 = 0.f;
   igso3_series_run<1>(st, kap, kapp, cexp, L - 1, L);
-  return SeriesAcc{st.b + st.b2, st.bp + st.bp2};
+  return SeriesAcc{st.b + st.b2, series_dF(kapp, st.bp + st.bp2)};
 }
 
 // ------------------------------------------------------------------------------------------------
