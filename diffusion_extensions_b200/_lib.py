@@ -51,6 +51,10 @@ SIGNATURES = {
     "so3d_se3_q_sample_f32": [_c_f, _c_f, _c_f, _c_f, _c_f, _i64, _c_f, _c_f, _c_f, ctypes.c_float, _u64, _u64, _u64, _c_f, _c_f, _c_f, _c_f, _i64, _c_f],
     "so3d_se3_p_sample_f32": [_c_f, _c_f, _c_f, _c_f, _c_f, _int, _c_f, _c_f, _c_f, _c_f, _c_f, _i64, _c_f, _c_f, _c_f, ctypes.c_float, _u64, _u64,
                               _u64, _c_f, _c_f, _i64, _c_f],
+    "so3d_se3_q_sample_dseed_f32": [_c_f, _c_f, _c_f, _c_f, _c_f, _i64, _c_f, _c_f, _c_f, ctypes.c_float, _c_f, _u64, _u64, _c_f, _c_f, _c_f, _c_f,
+                                    _i64, _c_f],
+    "so3d_se3_p_sample_dseed_f32": [_c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _i64, _c_f, _c_f, ctypes.c_float, _c_f, _u64, _u64,
+                                    _c_f, _c_f, _i64, _c_f],
     "so3d_bingham_sample_f32": [_c_f, _c_f, _u64, _u64, _u64, _c_f, _c_f, _i64, _c_f],
     "so3d_rotpredict_pack_f32": [_c_f] * 11 + [_c_f],
     "so3d_rotpredict_p_sample_f32": [_c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _i64, _c_f, _c_f, _u64, _u64, _u64, _c_f, _c_f, _i64, _c_f],

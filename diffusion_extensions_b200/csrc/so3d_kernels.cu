@@ -2130,10 +2130,29 @@ struct PStep2wOp : PStep2Op<kDevSeed> {
 // ------------------------------------------------------------------------------------------------
 constexpr uint64_t kShiftStream = 0x8000000000000000ull;
 
+// kDevSeed of the SE(3) ops: the Philox seed is read from device memory when the kernel runs (so3d_se3_*_dseed_f32: a
+// captured training step or sampling loop draws fresh noise on every replay).  Both streams come from it, the rotation
+// block at (row, rng_offset) and the translation block at (row, rng_offset | 2^63): the draws of the by-value kernels at
+// seed = *seed_dev.  The by-value instantiations derive from the empty DevSeedArgs<false>, so their layout and code are
+// those of the plain structs.
+template <bool kDevSeed>
+struct DevSeedArgs {};
+template <>
+struct DevSeedArgs<true> {
+  const uint64_t* seed_dev;
+  uint64_t rng_offset;
+  __device__ uint64_t load_seed() const { return (uint64_t)__ldg(reinterpret_cast<const unsigned long long*>(seed_dev)); }
+};
+// the seed a shared-t reverse step staged next to its scalars (two words after the six of the SE(3) step)
+__device__ __forceinline__ uint64_t staged_seed(const float* tab) {
+  return (uint64_t)__float_as_uint(tab[kTabScal + 6]) | ((uint64_t)__float_as_uint(tab[kTabScal + 7]) << 32);
+}
+
 // q_sample + p_losses targets: diffusion.py:498-516
 //   rot_t = so3_scale(rot0, a_t) @ noise_rot;  target_rot = vee(log noise_rot)/eps_t
 //   shift_t = a_t shift0 + eps_t shift_scale z;  target_shift = noise_shift/(eps_t shift_scale) = z
-struct SE3QSampleOp {
+template <bool kDevSeed = false>
+struct SE3QSampleOp : DevSeedArgs<kDevSeed> {
   SO3D_OP_ARRAYS_S(1, 1, 1, 3, 1)  // in: rot0 | shift0;  out: rot_t | target_rot, shift_t, target_shift
   static constexpr int kTab = kGrid;
   static constexpr bool kWarpSchedule = true;
@@ -2152,6 +2171,15 @@ struct SE3QSampleOp {
   PhiloxKey key, key_shift;  // (seed, rng_offset) and its translation stream (rng_offset | 2^63), built by the launcher
   uint64_t row_offset;
   __device__ void setup(float* tab) const { stage_cdf(tab, nullptr, loc); }
+  // the rotation draw and the translation block of global row r
+  __device__ NoiseDraw rot_draw(uint64_t r) const {
+    if constexpr (kDevSeed) return draw_axis_u(this->load_seed(), r, this->rng_offset);
+    else return draw_axis_u(key, r);
+  }
+  __device__ U4 shift_block(uint64_t r) const {
+    if constexpr (kDevSeed) return philox4x32_10(this->load_seed(), r, this->rng_offset | kShiftStream);
+    else return philox4x32_10(key_shift, r);
+  }
 #ifndef SO3D_SE3QS_PREFETCH
 #define SO3D_SE3QS_PREFETCH 1  // the software pipeline of QSampleOp: t two tiles ahead, draw + schedule scalars + guide record one tile ahead
 #endif
@@ -2172,7 +2200,7 @@ struct SE3QSampleOp {
     p.ti = (int)ti;
     p.eps = __ldg(sqrt_1m_ac + ti);
     p.sc = __ldg(sqrt_ac + ti);
-    p.d = draw_axis_u(key, row_offset + (uint64_t)i);
+    p.d = rot_draw(row_offset + (uint64_t)i);
     p.rec = guide ? __ldg(reinterpret_cast<const uint4*>(guide) + ti * kGuideRecs + guide_bucket(p.d.u)) : make_uint4(0, 0, 0, 0);
     return p;
   }
@@ -2191,7 +2219,7 @@ struct SE3QSampleOp {
     int64_t ti = t[i];
     ti = ti < 0 ? 0 : (ti >= T ? T - 1 : ti);
     const float eps = __ldg(sqrt_1m_ac + ti), sc = __ldg(sqrt_ac + ti);
-    const NoiseDraw d = draw_axis_u(key, row_offset + (uint64_t)i);
+    const NoiseDraw d = rot_draw(row_offset + (uint64_t)i);
     const float ang = table_row_angle(cdf, guide, ti, tab, d.u);
 #endif
     const Quat qn = quat_axis_angle(d.axis, ang);
@@ -2199,7 +2227,7 @@ struct SE3QSampleOp {
     o9[0] = quat_to_mat_unit(qmul(quat_axis_angle(ax.axis, sc * ax.theta), qn));
     const float k = ang * rcp_approx(eps);
     o3[0] = Vec3{k * d.axis.x, k * d.axis.y, k * d.axis.z};
-    const Normal4 z = normal4_from_u4(philox4x32_10(key_shift, row_offset + (uint64_t)i));
+    const Normal4 z = normal4_from_u4(shift_block(row_offset + (uint64_t)i));
     const float ns = eps * shift_scale;
     o3[1] = Vec3{fmaf(sc, a3[0].x, ns * z.a), fmaf(sc, a3[0].y, ns * z.b), fmaf(sc, a3[0].z, ns * z.c)};
     o3[2] = Vec3{z.a, z.b, z.c};
@@ -2218,16 +2246,19 @@ struct SE3QSampleOp {
 #ifndef SO3D_SE3QS2_INSTAGES
 #define SO3D_SE3QS2_INSTAGES 1
 #endif
-struct SE3QSample2Op : SE3QSampleOp {
+template <bool kDevSeed = false>
+struct SE3QSample2Op : SE3QSampleOp<kDevSeed> {
+  using Base = SE3QSampleOp<kDevSeed>;
+  using Pre2 = typename Base::Pre2;
   static constexpr int kMinCtas = SO3D_SE3QS2_MINCTAS;
   static constexpr int kInStages = SO3D_SE3QS2_INSTAGES;
   static constexpr bool kBranchless = SO3D_SE3QS2_BRANCHLESS;
   __device__ float angle_of(const Pre2& p, const float* tab) const {
-    if (guide) {
+    if (this->guide) {
       const GuideRec rec{p.rec.x, __uint_as_float(p.rec.y), __uint_as_float(p.rec.z), __uint_as_float(p.rec.w)};
-      return igso3_angle_from_record(cdf + (int64_t)p.ti * kCdf, tab + kTabLoc, rec, p.d.u);
+      return igso3_angle_from_record(this->cdf + (int64_t)p.ti * kCdf, tab + kTabLoc, rec, p.d.u);
     }
-    return igso3_angle_from_uniform(cdf + (int64_t)p.ti * kCdf, tab + kTabLoc, p.d.u);
+    return igso3_angle_from_uniform(this->cdf + (int64_t)p.ti * kCdf, tab + kTabLoc, p.d.u);
   }
   __device__ void row2(int64_t i0, const Pre2 (&p)[2], const Mat3 (*a9)[2], const Vec3 (*a3)[2], Mat3 (*o9)[2], Vec3 (*o3)[2], const float* tab) const {
     const L2 ang{angle_of(p[0], tab), angle_of(p[1], tab)};
@@ -2244,9 +2275,9 @@ struct SE3QSample2Op : SE3QSampleOp {
     const L2 tx = mul(kk, axis.x), ty = mul(kk, axis.y), tz = mul(kk, axis.z);
     o3[0][0] = Vec3{tx.x, ty.x, tz.x};
     o3[0][1] = Vec3{tx.y, ty.y, tz.y};
-    const Normal4 z0 = normal4_from_u4(philox4x32_10(key_shift, row_offset + (uint64_t)i0));
-    const Normal4 z1 = normal4_from_u4(philox4x32_10(key_shift, row_offset + (uint64_t)i0 + 32u));
-    const L2 ns = mul(eps, bc<L2>(shift_scale));
+    const Normal4 z0 = normal4_from_u4(this->shift_block(this->row_offset + (uint64_t)i0));
+    const Normal4 z1 = normal4_from_u4(this->shift_block(this->row_offset + (uint64_t)i0 + 32u));
+    const L2 ns = mul(eps, bc<L2>(this->shift_scale));
     const L2 sx = fma(sc, L2{a3[0][0].x, a3[0][1].x}, mul(ns, L2{z0.a, z1.a}));
     const L2 sy = fma(sc, L2{a3[0][0].y, a3[0][1].y}, mul(ns, L2{z0.b, z1.b}));
     const L2 sz = fma(sc, L2{a3[0][0].z, a3[0][1].z}, mul(ns, L2{z0.c, z1.c}));
@@ -2278,8 +2309,10 @@ struct SE3PStepPre<true> {
     uint4 rec;
   };
 };
-template <bool kSharedT>
-struct SE3PStepOp : SE3PStepPre<SO3D_SE3PS_PREFETCH && !kSharedT> {
+// kDevSeed (shared t only): the seed is read from seed_dev once per CTA in setup and staged next to the step's scalars.
+template <bool kSharedT, bool kDevSeed = false>
+struct SE3PStepOp : SE3PStepPre<SO3D_SE3PS_PREFETCH && !kSharedT>, DevSeedArgs<kDevSeed> {
+  static_assert(kSharedT || !kDevSeed, "the device-seed reverse step takes a shared step index");
   SO3D_OP_ARRAYS_S(1, 3, 1, 1, 1)  // in: rot_t | pred_rot, shift_t, pred_shift;  out: rot | shift
   static constexpr int kTab = kSharedT ? kTabCdfFloats : kGrid;
   // per-row t: cap SO3D_PS_MINCTAS (measured there).  Shared t: issue-bound, shared memory
@@ -2310,7 +2343,21 @@ struct SE3PStepOp : SE3PStepPre<SO3D_SE3PS_PREFETCH && !kSharedT> {
       tab[kTabScal + 3] = coef1[ti];
       tab[kTabScal + 4] = coef2[ti];
       tab[kTabScal + 5] = sigma[ti];
+      if constexpr (kDevSeed) {
+        const uint64_t sd = *this->seed_dev;
+        tab[kTabScal + 6] = __uint_as_float((uint32_t)sd);
+        tab[kTabScal + 7] = __uint_as_float((uint32_t)(sd >> 32));
+      }
     }
+  }
+  // the rotation draw and the translation block of global row r (kDevSeed: from the staged seed)
+  __device__ NoiseDraw rot_draw(uint64_t r, const float* tab) const {
+    if constexpr (kDevSeed) return draw_axis_u(staged_seed(tab), r, this->rng_offset);
+    else return draw_axis_u(key, r);
+  }
+  __device__ U4 shift_block(uint64_t r, const float* tab) const {
+    if constexpr (kDevSeed) return philox4x32_10(staged_seed(tab), r, this->rng_offset | kShiftStream);
+    else return philox4x32_10(key_shift, r);
   }
   __device__ void row(int64_t i, const Mat3* a9, const Vec3* a3, Mat3* o9, Vec3* o3, const float* tab) const {
     int64_t ti;
@@ -2330,10 +2377,10 @@ struct SE3PStepOp : SE3PStepPre<SO3D_SE3PS_PREFETCH && !kSharedT> {
     m.y = fmaf(k_c1, fmaf(k_recip, st.y, -k_recipm1 * ps.y), k_c2 * st.y);
     m.z = fmaf(k_c1, fmaf(k_recip, st.z, -k_recipm1 * ps.z), k_c2 * st.z);
     if (post_cdf && ti != 0) {
-      const NoiseDraw d = draw_axis_u(key, row_offset + (uint64_t)i);
+      const NoiseDraw d = rot_draw(row_offset + (uint64_t)i, tab);
       const float ang = kSharedT ? shared_row_angle(tab, d.u) : table_row_angle(post_cdf, post_guide, ti, tab, d.u);
       qm = qmul(qm, quat_axis_angle(d.axis, ang));
-      const Normal4 z = normal4_from_u4(philox4x32_10(key_shift, row_offset + (uint64_t)i));
+      const Normal4 z = normal4_from_u4(shift_block(row_offset + (uint64_t)i, tab));
       const float ns = k_sigma * shift_scale;
       m = Vec3{fmaf(ns, z.a, m.x), fmaf(ns, z.b, m.y), fmaf(ns, z.c, m.z)};
     }
@@ -2385,7 +2432,8 @@ struct SE3PStepOp : SE3PStepPre<SO3D_SE3PS_PREFETCH && !kSharedT> {
 #ifndef SO3D_SE3PS2_MINCTAS
 #define SO3D_SE3PS2_MINCTAS 5
 #endif
-struct SE3PStep2Op {
+template <bool kDevSeed = false>
+struct SE3PStep2Op : DevSeedArgs<kDevSeed> {
   SO3D_OP_ARRAYS_S(1, 3, 1, 1, 1)  // in: rot_t | pred_rot, shift_t, pred_shift;  out: rot | shift
   static constexpr int kTab = kTabCdfFloats;
   static constexpr int kMinCtas = SO3D_SE3PS2_MINCTAS;
@@ -2413,7 +2461,21 @@ struct SE3PStep2Op {
       tab[kTabScal + 3] = coef1[ti];
       tab[kTabScal + 4] = coef2[ti];
       tab[kTabScal + 5] = sigma ? sigma[ti] : 0.f;
+      if constexpr (kDevSeed) {
+        const uint64_t sd = *this->seed_dev;
+        tab[kTabScal + 6] = __uint_as_float((uint32_t)sd);
+        tab[kTabScal + 7] = __uint_as_float((uint32_t)(sd >> 32));
+      }
     }
+  }
+  // the rotation and translation blocks of global row r (kDevSeed: from the staged seed)
+  __device__ U4 rot_block(uint64_t r, const float* tab) const {
+    if constexpr (kDevSeed) return philox4x32_10(staged_seed(tab), r, this->rng_offset);
+    else return philox4x32_10(key, r);
+  }
+  __device__ U4 shift_block(uint64_t r, const float* tab) const {
+    if constexpr (kDevSeed) return philox4x32_10(staged_seed(tab), r, this->rng_offset | kShiftStream);
+    else return philox4x32_10(key_shift, r);
   }
   __device__ void row2(int64_t i0, const Mat3 (*a9)[2], const Vec3 (*a3)[2], Mat3 (*o9)[2], Vec3 (*o3)[2], const float* tab) const {
     const int ti = __float_as_int(tab[kTabScal]);
@@ -2431,11 +2493,11 @@ struct SE3PStep2Op {
                 fma(c1, fma(rc, st.z, mul(nrm1, ps.z)), mul(c2, st.z))};
     if (post_cdf && ti != 0) {
       const uint64_t row = row_offset + (uint64_t)i0;
-      const U4 r0 = philox4x32_10(key, row), r1 = philox4x32_10(key, row + kT2);
+      const U4 r0 = rot_block(row, tab), r1 = rot_block(row + kT2, tab);
       const Vec3L<L2> axis = sphere_from_uniforms_l(L2{u01(r0.x), u01(r1.x)}, L2{u01(r0.y), u01(r1.y)});
       const L2 ang{shared_row_angle(tab, u01(r0.z)), shared_row_angle(tab, u01(r1.z))};
       qm = qmul_l(qm, quat_axis_angle_l(axis, ang));
-      const Normal4 z0 = normal4_from_u4(philox4x32_10(key_shift, row)), z1 = normal4_from_u4(philox4x32_10(key_shift, row + kT2));
+      const Normal4 z0 = normal4_from_u4(shift_block(row, tab)), z1 = normal4_from_u4(shift_block(row + kT2, tab));
       const L2 ns = bc<L2>(k_sigma * shift_scale);
       m = Vec3L<L2>{fma(ns, L2{z0.a, z1.a}, m.x), fma(ns, L2{z0.b, z1.b}, m.y), fma(ns, L2{z0.c, z1.c}, m.z)};
     }
@@ -2895,21 +2957,64 @@ int so3d_p_sample_dseed_f32(const float* x_t, const float* pred3, const int64_t*
 
 }  // extern "C"
 
-template <bool kSharedT>
+template <bool kSharedT, bool kDevSeed = false>
 static int launch_se3_p_step(const float* rot_t, const float* shift_t, const float* pred_rot3, const float* pred_shift3, const int64_t* t,
                              const float* recip, const float* recipm1, const float* coef1, const float* coef2, const float* sigma, int64_t T,
                              const float* post_cdf, const uint32_t* post_guide, const float* loc, float shift_scale, uint64_t seed,
-                             uint64_t rng_offset, uint64_t row_offset, float* rot_out, float* shift_out, int64_t n, void* stream) {
-  SE3PStepOp<kSharedT> op;
-  op.in9[0] = rot_t; op.in3[0] = pred_rot3; op.in3[1] = shift_t; op.in3[2] = pred_shift3; op.out9[0] = rot_out; op.out3[0] = shift_out;
-  op.t = t; op.recip = recip; op.recipm1 = recipm1; op.coef1 = coef1; op.coef2 = coef2; op.sigma = sigma; op.T = T;
-  op.post_cdf = post_cdf; op.post_guide = post_guide; op.loc = loc; op.shift_scale = shift_scale;
-  op.key = make_philox_key(seed, rng_offset); op.key_shift = make_philox_key(seed, rng_offset | kShiftStream); op.row_offset = row_offset;
-  if constexpr (!kSharedT) {  // per-row t (r05d, r05f)
-    if constexpr (SO3D_SE3PS_PREFETCH) return launch_rowwise_pick_pre(op, n, stream, "so3d_se3_p_sample_f32", SO3D_SE3PS_ROWS_TWO != 0);
-    else return launch_rowwise_pick(op, n, stream, "so3d_se3_p_sample_f32", SO3D_SE3PS_ROWS_TWO != 0);
+                             uint64_t rng_offset, uint64_t row_offset, float* rot_out, float* shift_out, int64_t n, void* stream,
+                             const uint64_t* seed_dev = nullptr) {
+  const char* name = kDevSeed ? "so3d_se3_p_sample_dseed_f32" : "so3d_se3_p_sample_f32";
+  auto fill = [&](auto& op) {
+    if constexpr (kDevSeed) op.seed_dev = seed_dev, op.rng_offset = rng_offset;
+    op.in9[0] = rot_t; op.in3[0] = pred_rot3; op.in3[1] = shift_t; op.in3[2] = pred_shift3; op.out9[0] = rot_out; op.out3[0] = shift_out;
+    op.t = t; op.recip = recip; op.recipm1 = recipm1; op.coef1 = coef1; op.coef2 = coef2; op.sigma = sigma; op.T = T;
+    op.post_cdf = post_cdf; op.loc = loc; op.shift_scale = shift_scale;
+    op.key = make_philox_key(seed, rng_offset); op.key_shift = make_philox_key(seed, rng_offset | kShiftStream); op.row_offset = row_offset;
+  };
+  if constexpr (kSharedT) {
+    // the shared-t step with noise: two rows per thread by default (SO3D_SE3_PSTEP_LANES=1 selects the one-row kernel, A/B aid)
+    static const bool one_lane = [] { const char* e = getenv("SO3D_SE3_PSTEP_LANES"); return e && atoi(e) == 1; }();
+    if (!one_lane && post_cdf) {
+      SE3PStep2Op<kDevSeed> op;
+      fill(op);
+      return launch_rowwise2(op, n, stream, name);
+    }
   }
-  return launch_rowwise(op, n, stream, "so3d_se3_p_sample_f32");
+  SE3PStepOp<kSharedT, kDevSeed> op;
+  fill(op);
+  op.post_guide = post_guide;
+  if constexpr (!kSharedT) {  // per-row t (r05d, r05f)
+    if constexpr (SO3D_SE3PS_PREFETCH) return launch_rowwise_pick_pre(op, n, stream, name, SO3D_SE3PS_ROWS_TWO != 0);
+    else return launch_rowwise_pick(op, n, stream, name, SO3D_SE3PS_ROWS_TWO != 0);
+  }
+  return launch_rowwise(op, n, stream, name);
+}
+
+template <bool kDevSeed>
+static int launch_se3_q_sample(const float* rot0, const float* shift0, const int64_t* t, const float* sqrt_ac, const float* sqrt_1m_ac,
+                               int64_t T, const float* cdf, const uint32_t* guide, const float* loc, float shift_scale, uint64_t seed,
+                               uint64_t rng_offset, uint64_t row_offset, float* rot_t, float* shift_t, float* target_rot3,
+                               float* target_shift3, int64_t n, void* stream, const uint64_t* seed_dev = nullptr) {
+  const char* name = kDevSeed ? "so3d_se3_q_sample_dseed_f32" : "so3d_se3_q_sample_f32";
+  auto fill = [&](auto& op) {
+    if constexpr (kDevSeed) op.seed_dev = seed_dev, op.rng_offset = rng_offset;
+    op.in9[0] = rot0; op.in3[0] = shift0; op.out9[0] = rot_t; op.out3[0] = target_rot3; op.out3[1] = shift_t; op.out3[2] = target_shift3;
+    op.t = t; op.sqrt_ac = sqrt_ac; op.sqrt_1m_ac = sqrt_1m_ac; op.T = T; op.cdf = cdf; op.guide = guide; op.loc = loc;
+    op.shift_scale = shift_scale; op.key = make_philox_key(seed, rng_offset); op.key_shift = make_philox_key(seed, rng_offset | kShiftStream); op.row_offset = row_offset;
+  };
+#if SO3D_SE3QS_PREFETCH
+  // Two rows per thread with per-warp input slices: 0.424 -> 0.412 ms (r04k; with the CTA-wide input ring it was no faster,
+  // r04f/r04g).  SO3D_SE3_QS_LANES=1 selects the one-row kernel (cross-kernel parity test).
+  const char* lanes_env = getenv("SO3D_SE3_QS_LANES");
+  if (!(lanes_env && atoi(lanes_env) == 1)) {
+    SE3QSample2Op<kDevSeed> op2;
+    fill(op2);
+    return launch_rowwise_w2(op2, n, stream, name);
+  }
+#endif
+  SE3QSampleOp<kDevSeed> op;
+  fill(op);
+  return launch_rowwise(op, n, stream, name);
 }
 
 extern "C" {
@@ -2923,24 +3028,22 @@ int so3d_se3_q_sample_f32(const float* rot0, const float* shift0, const int64_t*
   SO3D_REQUIRE(rot0 && shift0 && t && sqrt_ac && sqrt_1m_ac && cdf && loc && rot_t && shift_t, "so3d_se3_q_sample_f32: null pointer");
   SO3D_REQUIRE(T > 0, "so3d_se3_q_sample_f32: T must be positive");
   SO3D_REQUIRE(rng_offset < kShiftStream, "so3d_se3_q_sample_f32: rng_offset must be below 2^63");
-  auto fill = [&](auto& op) {
-    op.in9[0] = rot0; op.in3[0] = shift0; op.out9[0] = rot_t; op.out3[0] = target_rot3; op.out3[1] = shift_t; op.out3[2] = target_shift3;
-    op.t = t; op.sqrt_ac = sqrt_ac; op.sqrt_1m_ac = sqrt_1m_ac; op.T = T; op.cdf = cdf; op.guide = guide; op.loc = loc;
-    op.shift_scale = shift_scale; op.key = make_philox_key(seed, rng_offset); op.key_shift = make_philox_key(seed, rng_offset | kShiftStream); op.row_offset = row_offset;
-  };
-#if SO3D_SE3QS_PREFETCH
-  // Two rows per thread with per-warp input slices: 0.424 -> 0.412 ms (r04k; with the CTA-wide input ring it was no faster,
-  // r04f/r04g).  SO3D_SE3_QS_LANES=1 selects the one-row kernel (cross-kernel parity test).
-  const char* lanes_env = getenv("SO3D_SE3_QS_LANES");
-  if (!(lanes_env && atoi(lanes_env) == 1)) {
-    SE3QSample2Op op2;
-    fill(op2);
-    return launch_rowwise_w2(op2, n, stream, "so3d_se3_q_sample_f32");
-  }
-#endif
-  SE3QSampleOp op;
-  fill(op);
-  return launch_rowwise(op, n, stream, "so3d_se3_q_sample_f32");
+  return launch_se3_q_sample<false>(rot0, shift0, t, sqrt_ac, sqrt_1m_ac, T, cdf, guide, loc, shift_scale, seed, rng_offset, row_offset, rot_t,
+                                    shift_t, target_rot3, target_shift3, n, stream);
+}
+
+int so3d_se3_q_sample_dseed_f32(const float* rot0, const float* shift0, const int64_t* t, const float* sqrt_ac, const float* sqrt_1m_ac,
+                                int64_t T, const float* cdf, const uint32_t* guide, const float* loc, float shift_scale,
+                                const uint64_t* seed_dev, uint64_t rng_offset, uint64_t row_offset, float* rot_t, float* shift_t,
+                                float* target_rot3, float* target_shift3, int64_t n, void* stream) {
+  SO3D_REQUIRE(n >= 0, "negative n");
+  if (n == 0) return 0;
+  SO3D_REQUIRE(rot0 && shift0 && t && sqrt_ac && sqrt_1m_ac && cdf && loc && rot_t && shift_t && seed_dev,
+               "so3d_se3_q_sample_dseed_f32: null pointer");
+  SO3D_REQUIRE(T > 0, "so3d_se3_q_sample_dseed_f32: T must be positive");
+  SO3D_REQUIRE(rng_offset < kShiftStream, "so3d_se3_q_sample_dseed_f32: rng_offset must be below 2^63");
+  return launch_se3_q_sample<true>(rot0, shift0, t, sqrt_ac, sqrt_1m_ac, T, cdf, guide, loc, shift_scale, 0, rng_offset, row_offset, rot_t,
+                                   shift_t, target_rot3, target_shift3, n, stream, seed_dev);
 }
 
 int so3d_se3_p_sample_f32(const float* rot_t, const float* shift_t, const float* pred_rot3, const float* pred_shift3, const int64_t* t,
@@ -2956,21 +3059,26 @@ int so3d_se3_p_sample_f32(const float* rot_t, const float* shift_t, const float*
   SO3D_REQUIRE(t_stride == 0 || t_stride == 1, "t_stride must be 0 or 1");
   SO3D_REQUIRE(!post_cdf || (loc && sigma), "so3d_se3_p_sample_f32: loc and sigma required with post_cdf");
   SO3D_REQUIRE(rng_offset < kShiftStream, "so3d_se3_p_sample_f32: rng_offset must be below 2^63");
-  if (t_stride == 0) {
-    static const bool one_lane = [] { const char* e = getenv("SO3D_SE3_PSTEP_LANES"); return e && atoi(e) == 1; }();  // A/B aid
-    if (!one_lane && post_cdf) {
-      SE3PStep2Op op;
-      op.in9[0] = rot_t; op.in3[0] = pred_rot3; op.in3[1] = shift_t; op.in3[2] = pred_shift3; op.out9[0] = rot_out; op.out3[0] = shift_out;
-      op.t = t; op.recip = recip; op.recipm1 = recipm1; op.coef1 = coef1; op.coef2 = coef2; op.sigma = sigma; op.T = T;
-      op.post_cdf = post_cdf; op.loc = loc; op.shift_scale = shift_scale;
-      op.key = make_philox_key(seed, rng_offset); op.key_shift = make_philox_key(seed, rng_offset | kShiftStream); op.row_offset = row_offset;
-      return launch_rowwise2(op, n, stream, "so3d_se3_p_sample_f32");
-    }
+  if (t_stride == 0)
     return launch_se3_p_step<true>(rot_t, shift_t, pred_rot3, pred_shift3, t, recip, recipm1, coef1, coef2, sigma, T, post_cdf, post_guide, loc,
                                    shift_scale, seed, rng_offset, row_offset, rot_out, shift_out, n, stream);
-  }
   return launch_se3_p_step<false>(rot_t, shift_t, pred_rot3, pred_shift3, t, recip, recipm1, coef1, coef2, sigma, T, post_cdf, post_guide, loc,
                                   shift_scale, seed, rng_offset, row_offset, rot_out, shift_out, n, stream);
+}
+
+int so3d_se3_p_sample_dseed_f32(const float* rot_t, const float* shift_t, const float* pred_rot3, const float* pred_shift3, const int64_t* t,
+                                const float* recip, const float* recipm1, const float* coef1, const float* coef2, const float* sigma,
+                                int64_t T, const float* post_cdf, const float* loc, float shift_scale, const uint64_t* seed_dev,
+                                uint64_t rng_offset, uint64_t row_offset, float* rot_out, float* shift_out, int64_t n, void* stream) {
+  SO3D_REQUIRE(n >= 0, "negative n");
+  if (n == 0) return 0;
+  SO3D_REQUIRE(rot_t && shift_t && pred_rot3 && pred_shift3 && t && recip && recipm1 && coef1 && coef2 && sigma && post_cdf && loc && seed_dev &&
+                   rot_out && shift_out,
+               "so3d_se3_p_sample_dseed_f32: null pointer");
+  SO3D_REQUIRE(T > 0, "so3d_se3_p_sample_dseed_f32: T must be positive");
+  SO3D_REQUIRE(rng_offset < kShiftStream, "so3d_se3_p_sample_dseed_f32: rng_offset must be below 2^63");
+  return launch_se3_p_step<true, true>(rot_t, shift_t, pred_rot3, pred_shift3, t, recip, recipm1, coef1, coef2, sigma, T, post_cdf, nullptr, loc,
+                                       shift_scale, 0, rng_offset, row_offset, rot_out, shift_out, n, stream, seed_dev);
 }
 
 }  // extern "C"

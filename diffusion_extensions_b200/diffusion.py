@@ -159,9 +159,10 @@ class SO3Diffusion(nn.Module):
 
     def make_graphed_train_step(self, optimizer, example_x, warmup=3, sync_grads=None):
         """so3_train.py:70-76 / bingham_train.py:88-95 as ONE CUDA graph: `loss = self(x); loss.backward(); optimizer.step()`
-        is captured once for batches shaped like `example_x` (the optimizer must be constructed with capturable=True) and
-        the returned `step(x) -> loss` copies x into the graph's input and replays it.  At the reference's batch sizes the
-        eager step is launch-bound (~50 launches, 1.05 ms); the replay takes 0.18 ms at batch 256 (tests/tools/probe_train.py).
+        is captured once for batches shaped like `example_x` (a tensor, or an `AffineT` for the SE(3) classes; the optimizer
+        must be constructed with capturable=True) and the returned `step(x) -> loss` copies x into the graph's input and
+        replays it.  At the reference's batch sizes the eager step is launch-bound (~50 launches, 1.05 ms); the replay takes
+        0.18 ms at batch 256 (tests/tools/probe_train.py).
         Noise comes from the device-resident seed (use_device_seed), step indices from torch's graph-safe generator.
 
         Data-parallel training (BASELINE cfg 4): with `sync_grads` (default: a process group with more than one rank is
@@ -309,7 +310,8 @@ class SO3Diffusion(nn.Module):
         """Capture the T launches of the loop once per (batch shape, denoiser, weights) and replay them: the loop is
         launch-bound for the batch sizes the reference samples (bingham_test.py:25, 20 000 particles: ~10 us of GPU work
         per step), and a replay costs one launch.  Noise differs between replays because the kernels read the seed
-        from `seed_buf` when they run (so3d_p_sample_dseed_f32 / so3d_rotpredict_p_sample_dseed_f32)."""
+        from `seed_buf` when they run (so3d_p_sample_dseed_f32 / so3d_rotpredict_p_sample_dseed_f32; the SE(3) classes
+        supply their own step through `_p_sample_seeded`: so3d_se3_p_sample_dseed_f32)."""
         dev = x.device
         fn = self.denoise_fn
         probe = self._fused_denoiser(x, self.tables()[2][:1])          # (re)packs the weights if they changed
@@ -482,10 +484,15 @@ class SE3Diffusion(SO3Diffusion):
 
     def noise_and_target(self, x_start: AffineT, t):
         """One fused launch: noise ~ IGSO3xR3(eps_t, shift_scale), x_t, and both 'grad_mse' targets
-        (diffusion.py:508-516).  -> (x_t: AffineT, target: AffineGrad)"""
+        (diffusion.py:508-516).  -> (x_t: AffineT, target: AffineGrad)
+        With `use_device_seed` the seed lives on the device and is bumped there before the launch (capturable)."""
         fwd, _, _ = self.tables()
+        dseed = self.__dict__.get("_device_seed")
+        if dseed is not None:
+            dseed.add_(1)                                    # a captured kernel: every replay uses the next seed
         out = ops.se3_q_sample_fused(x_start.rot, x_start.shift, t, self.sqrt_alphas_cumprod, self.sqrt_one_minus_alphas_cumprod, fwd,
-                                     self.shift_scale, row_offset=self.row_offset, guide=self.guides()[0])
+                                     self.shift_scale, seed=dseed, rng_offset=0 if dseed is not None else None, row_offset=self.row_offset,
+                                     guide=self.guides()[0])
         return AffineT(out["rot"], out["shift"]), AffineGrad(out["target_rot"], out["target_shift"])
 
     def q_sample(self, x_start: AffineT, t, noise: AffineT = None):
@@ -531,15 +538,30 @@ class SE3Diffusion(SO3Diffusion):
         """diffusion.py:473-485: one fused kernel after the denoiser; rows with t == 0 get no noise (device-side check)."""
         return self._step(x, self._denoise(x, t), t, noise=True)
 
+    def _p_sample_seeded(self, x: AffineT, t, seed_buf, step):
+        """The step of the captured loop (SO3Diffusion._p_sample_loop_graph): the denoiser sees a (B,) step index as in the
+        eager loop, the kernel the shared step `t` with the seed read from `seed_buf` and rng_offset = step."""
+        _, post, _ = self.tables()
+        predict = self._denoise(x, torch.full(x.rot.shape[:1], step, device=x.device, dtype=torch.long))
+        rot, shift = ops.se3_p_sample_fused(x.rot, x.shift, predict.rot_g, predict.shift_g, t, *self._sched(), self._sigma(), self.shift_scale,
+                                            post_cdf=post, seed=seed_buf, rng_offset=step, row_offset=self.row_offset)
+        return AffineT(rot, shift)
+
     @torch.no_grad()
-    def p_sample_loop(self, shape, init="haar", progress=False):
+    def p_sample_loop(self, shape, init="haar", progress=False, cuda_graph=False):
         """diffusion.py:487-496 (the reference starts from rotations only; here the translation starts at
-        N(0, shift_scale^2 I), the forward process's terminal law, like ProjectedSE3Diffusion does with N(0, I))."""
+        N(0, shift_scale^2 I), the forward process's terminal law, like ProjectedSE3Diffusion does with N(0, I)).
+        cuda_graph=True replays the whole loop as one captured CUDA graph (same distribution, its own noise stream)."""
         device = self.betas.device
         shape = tuple(shape)
         x = AffineT(self._init_rot(shape, init), torch.randn(*shape, 3, device=device) * self.shift_scale)
+        return self._run_loop(x, shape, progress, cuda_graph)
+
+    def _run_loop(self, x: AffineT, shape, progress, cuda_graph):
+        if cuda_graph:
+            return self._p_sample_loop_graph(AffineT(x.rot.contiguous(), x.shift.contiguous()))
         for i in self._steps(progress):
-            x = self.p_sample(x, torch.full(shape[:1], i, device=device, dtype=torch.long))
+            x = self.p_sample(x, torch.full(shape[:1], i, device=x.device, dtype=torch.long))
         return x
 
     def _init_rot(self, shape, init):
@@ -586,15 +608,13 @@ class ProjectedSE3Diffusion(SE3Diffusion):
         return self.denoise_fn(self.projection(x), t)
 
     @torch.no_grad()
-    def p_sample_loop(self, shape, projection, init="haar", progress=False):
-        """diffusion.py:541-552: translation starts from N(0, I) as in the reference."""
+    def p_sample_loop(self, shape, projection, init="haar", progress=False, cuda_graph=False):
+        """diffusion.py:541-552: translation starts from N(0, I) as in the reference.  cuda_graph as in SE3Diffusion."""
         self.projection = projection
         device = self.betas.device
         shape = tuple(shape)
         x = AffineT(self._init_rot(shape, init), torch.randn(*shape, 3, device=device))
-        for i in self._steps(progress):
-            x = self.p_sample(x, torch.full(shape[:1], i, device=device, dtype=torch.long))
-        return x
+        return self._run_loop(x, shape, progress, cuda_graph)
 
     def forward(self, x: AffineT, projection, *args, **kwargs):
         self.projection = projection

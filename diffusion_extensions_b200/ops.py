@@ -473,7 +473,8 @@ def _rows_t(t, bs, dev):
 
 def se3_q_sample_fused(rot0, shift0, t, sqrt_ac, sqrt_1m_ac, cdf, shift_scale, seed=None, rng_offset=None, row_offset=0,
                        want_target=True, guide=None):
-    """-> dict(rot, shift, target_rot, target_shift)."""
+    """-> dict(rot, shift, target_rot, target_shift).  seed: an int with rng_offset (by value), None (the module's Philox
+    stream), or a one-element int64 device tensor read when the kernel runs (CUDA-graph replays; rng_offset required)."""
     rot0, bs, n = _rows9(rot0, "x_start.rot")
     dev = rot0.device
     shift0 = check_f32(shift0, "x_start.shift", (3,)).expand(*bs, 3).contiguous()
@@ -486,11 +487,18 @@ def se3_q_sample_fused(rot0, shift0, t, sqrt_ac, sqrt_1m_ac, cdf, shift_scale, s
         raise ValueError("cdf table must have one row per timestep")
     _check_guide(guide, T, "guide")
     _, _, trap_loc = cdf_grid(dev)
-    if seed is None or rng_offset is None:
+    seed_dev = _seed_tensor(seed, dev)
+    if seed_dev is not None and rng_offset is None:
+        raise ValueError("a device seed needs an explicit rng_offset")
+    if seed_dev is None and (seed is None or rng_offset is None):
         seed, rng_offset = rng.next()
     rot_t, shift_t = torch.empty_like(rot0), torch.empty_like(shift0)
     tr = torch.empty_like(shift0) if want_target else None
     ts = torch.empty_like(shift0) if want_target else None
+    if seed_dev is not None:  # CUDA-graph replayable launch: the seed is read on the device when the kernel runs
+        call("so3d_se3_q_sample_dseed_f32", ptr(rot0), ptr(shift0), ptr(t), ptr(sqrt_ac), ptr(sqrt_1m_ac), T, ptr(cdf), ptr(guide), ptr(trap_loc),
+             float(shift_scale), ptr(seed_dev), int(rng_offset), int(row_offset), ptr(rot_t), ptr(shift_t), ptr(tr), ptr(ts), n, device=dev)
+        return {"rot": rot_t, "shift": shift_t, "target_rot": tr, "target_shift": ts}
     call("so3d_se3_q_sample_f32", ptr(rot0), ptr(shift0), ptr(t), ptr(sqrt_ac), ptr(sqrt_1m_ac), T, ptr(cdf), ptr(guide), ptr(trap_loc),
          float(shift_scale), seed, rng_offset, int(row_offset), ptr(rot_t), ptr(shift_t), ptr(tr), ptr(ts), n, device=dev)
     return {"rot": rot_t, "shift": shift_t, "target_rot": tr, "target_shift": ts}
@@ -499,7 +507,8 @@ def se3_q_sample_fused(rot0, shift0, t, sqrt_ac, sqrt_1m_ac, cdf, shift_scale, s
 def se3_p_sample_fused(rot_t, shift_t, pred_rot, pred_shift, t, recip, recipm1, coef1, coef2, sigma, shift_scale, post_cdf=None,
                        seed=None, rng_offset=None, row_offset=0, post_guide=None):
     """Fused SE(3) reverse step; t with one element = shared step.  post_cdf None -> posterior mean only.
-    -> (rot (...,3,3), shift (...,3))"""
+    seed may be a one-element int64 device tensor read when the kernel runs (CUDA-graph replays): that takes a shared
+    step, post_cdf and an explicit rng_offset.  -> (rot (...,3,3), shift (...,3))"""
     rot_t, bs, n = _rows9(rot_t, "x.rot")
     dev = rot_t.device
     shift_t = check_f32(shift_t, "x.shift", (3,)).expand(*bs, 3).contiguous()
@@ -521,9 +530,18 @@ def se3_p_sample_fused(rot_t, shift_t, pred_rot, pred_shift, t, recip, recipm1, 
             raise ValueError("posterior cdf table must have one row per timestep")
         _check_guide(post_guide, T, "post_guide")
         _, _, trap_loc = cdf_grid(dev)
-        if seed is None or rng_offset is None:
-            seed, rng_offset = rng.next()
+    seed_dev = _seed_tensor(seed, dev)
+    if seed_dev is not None:
+        if post_cdf is None or t_stride != 0 or rng_offset is None:
+            raise ValueError("a device seed needs a shared step index, post_cdf and an explicit rng_offset")
+    elif post_cdf is not None and (seed is None or rng_offset is None):
+        seed, rng_offset = rng.next()
     rot_out, shift_out = torch.empty_like(rot_t), torch.empty_like(shift_t)
+    if seed_dev is not None:  # CUDA-graph replayable step: the seed is read on the device when the kernel runs
+        call("so3d_se3_p_sample_dseed_f32", ptr(rot_t), ptr(shift_t), ptr(pred_rot), ptr(pred_shift), ptr(t), ptr(recip), ptr(recipm1), ptr(coef1),
+             ptr(coef2), ptr(sigma), T, ptr(post_cdf), ptr(trap_loc), float(shift_scale), ptr(seed_dev), int(rng_offset), int(row_offset),
+             ptr(rot_out), ptr(shift_out), n, device=dev)
+        return rot_out, shift_out
     call("so3d_se3_p_sample_f32", ptr(rot_t), ptr(shift_t), ptr(pred_rot), ptr(pred_shift), ptr(t), t_stride, ptr(recip), ptr(recipm1),
          ptr(coef1), ptr(coef2), ptr(sigma), T, ptr(post_cdf), ptr(post_guide), ptr(trap_loc), float(shift_scale), seed or 0, rng_offset or 0,
          int(row_offset), ptr(rot_out), ptr(shift_out), n, device=dev)

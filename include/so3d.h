@@ -226,6 +226,14 @@ int so3d_se3_q_sample_f32(const float* rot0, const float* shift0, const int64_t*
                           const float* sqrt_1m_ac, int64_t T, const float* cdf, const uint32_t* guide, const float* loc,
                           float shift_scale, uint64_t seed, uint64_t rng_offset, uint64_t row_offset, float* rot_t,
                           float* shift_t, float* target_rot3, float* target_shift3, int64_t n, void* stream);
+/* so3d_se3_q_sample_f32 with the Philox SEED READ FROM DEVICE MEMORY when the kernel runs: a captured SE(3) training
+ * step draws fresh rotation and translation noise on every replay after the caller bumps *seed_dev (a captured
+ * `seed.add_(1)`).  Both streams come from *seed_dev (rotation at rng_offset, translation at rng_offset | 2^63): the draws
+ * equal so3d_se3_q_sample_f32's at seed = *seed_dev.  target_rot3 / target_shift3 nullable.  rng_offset < 2^63. */
+int so3d_se3_q_sample_dseed_f32(const float* rot0, const float* shift0, const int64_t* t, const float* sqrt_ac,
+                                const float* sqrt_1m_ac, int64_t T, const float* cdf, const uint32_t* guide, const float* loc,
+                                float shift_scale, const uint64_t* seed_dev, uint64_t rng_offset, uint64_t row_offset,
+                                float* rot_t, float* shift_t, float* target_rot3, float* target_shift3, int64_t n, void* stream);
 /* diffusion.py:446-485 (SE3Diffusion.predict_start_from_noise, q_posterior, p_sample), fused.  Rotation half as
  * so3d_p_sample_f32; translation half
  *   shift0_hat = recip[t] shift_t - recipm1[t] pred_shift;  mean = coef1[t] shift0_hat + coef2[t] shift_t;
@@ -236,6 +244,15 @@ int so3d_se3_p_sample_f32(const float* rot_t, const float* shift_t, const float*
                           const float* coef2, const float* sigma, int64_t T, const float* post_cdf,
                           const uint32_t* post_guide, const float* loc, float shift_scale, uint64_t seed, uint64_t rng_offset,
                           uint64_t row_offset, float* rot_out, float* shift_out, int64_t n, void* stream);
+/* The same step (shared t: int64[1] on the device, noise on, post_cdf required) with the Philox SEED READ FROM DEVICE
+ * MEMORY at execution time: a captured CUDA graph of a whole SE(3) sampling loop (one launch per step with
+ * rng_offset = step) draws fresh noise on every replay once the caller has written a new seed to seed_dev.  Draws of
+ * both halves equal so3d_se3_p_sample_f32's at seed = *seed_dev.  rng_offset < 2^63. */
+int so3d_se3_p_sample_dseed_f32(const float* rot_t, const float* shift_t, const float* pred_rot3, const float* pred_shift3,
+                                const int64_t* t, const float* recip, const float* recipm1, const float* coef1,
+                                const float* coef2, const float* sigma, int64_t T, const float* post_cdf, const float* loc,
+                                float shift_scale, const uint64_t* seed_dev, uint64_t rng_offset, uint64_t row_offset,
+                                float* rot_out, float* shift_out, int64_t n, void* stream);
 
 /* ---- data side: distributions.py Bingham (SURVEY 8f-2) ------------------------------------------- */
 /* distributions.py:113-127 Bingham.rsample (zero-mean MultivariateNormal in R^4, normalised to a unit quaternion,
