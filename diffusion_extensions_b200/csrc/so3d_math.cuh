@@ -547,6 +547,13 @@ SO3D_HD Vec3 vee_adj(const Mat3& g) { return Vec3{g.m[7] - g.m[5], g.m[2] - g.m[
 //   dL = a * dscale + scale <GL - GL^T, dR>,   a = <GL, R - R^T>
 //   dscale = ds [ c/(2 s (s^2+c^2)) - theta/(2 s^2) ] - dc / (2 (s^2+c^2)),
 //   ds = <R - R^T, dR>/(4 s),  dc = tr(dR)/2.
+// For c < kNearPiCos the formula's component along SO(3) is ill-conditioned: R - R^T holds only ~2^-24 absolute
+// precision, and evaluated on an fp32 matrix (orthonormal to ~6e-8) the formula's tangent part is off by ~2^-24/sin^2(theta).
+// There the tangent component, vee_adj(R^T g), is replaced by the derivative of log along R exp(hat(xi)),
+//   Jr^-T(theta n) vee_adj(GL) = u - (theta/2) n x u + (1 - (theta/2) sin(theta)/(1 - cos(theta))) n x (n x u),
+// with theta and n from axis_angle's symmetric-part branch; the normal component (R times the symmetric part of R^T g)
+// stays the reference formula's.  The error of the tangent part is then ~2^-24/sin(theta), the rounding of the fp32
+// output, whose normal entries are of size 1/sin(theta).
 SO3D_HD Mat3 log_bwd(const Mat3& r, const Mat3& gl) {
   const float vx = r.m[7] - r.m[5], vy = r.m[2] - r.m[6], vz = r.m[3] - r.m[1];
   const float s = 0.5f * sqrtf(fmaf(vx, vx, fmaf(vy, vy, vz * vz)));
@@ -567,9 +574,10 @@ SO3D_HD Mat3 log_bwd(const Mat3& r, const Mat3& gl) {
     ks = (c / (2.0f * s * den) - th / (2.0f * s * s)) / (4.0f * s);
     kc = -1.0f / (4.0f * den);
   } else if (c > 0.f) {
-    // theta -> 0 limits: scale -> 1/2 + s^2/12 (orthonormal input), d scale/ds * 1/(4s) -> 1/24
+    // theta -> 0 limits: scale -> 1/2 + s^2/12 (orthonormal input); ks is the partial d scale/ds at fixed c, over 4 s,
+    // -> -1/(12 c^3) = -1/12 (the total derivative along SO(3), 1/24, is not what the chain rule above needs)
     scale = 0.5f + s * s * (1.0f / 12.0f);
-    ks = (1.0f / 24.0f);
+    ks = -(1.0f / 12.0f);
     kc = -1.0f / (4.0f * den);
   } else {
     // theta -> pi: the formula is singular (scale ~ pi/(2 s)); keep it finite, gradient is ill-defined
@@ -587,6 +595,21 @@ SO3D_HD Mat3 log_bwd(const Mat3& r, const Mat3& gl) {
       if (i == j) v = fmaf(ga, kc, v);
       g.m[3 * i + j] = v;
     }
+  if (c < kNearPiCos) {
+    const AxisAngle aa = axis_angle(r);
+    const Vec3 n = aa.axis, u = vee_adj(gl);
+    const float ht = 0.5f * aa.theta;
+    const float kq = 1.0f - ht * s / (1.0f - c);
+    const Vec3 nu{n.y * u.z - n.z * u.y, n.z * u.x - n.x * u.z, n.x * u.y - n.y * u.x};        // n x u
+    const Vec3 nnu{n.y * nu.z - n.z * nu.y, n.z * nu.x - n.x * nu.z, n.x * nu.y - n.y * nu.x};  // n x (n x u)
+    const Vec3 cur = vee_adj(mul_tn(r, g));
+    // g += R hat(d)/2 moves vee_adj(R^T g) by d
+    const Vec3 d{0.5f * (fmaf(kq, nnu.x, fmaf(-ht, nu.x, u.x)) - cur.x), 0.5f * (fmaf(kq, nnu.y, fmaf(-ht, nu.y, u.y)) - cur.y),
+                 0.5f * (fmaf(kq, nnu.z, fmaf(-ht, nu.z, u.z)) - cur.z)};
+    const Mat3 corr = mul_nn(r, hat(d));
+#pragma unroll
+    for (int k = 0; k < 9; ++k) g.m[k] += corr.m[k];
+  }
   return g;
 }
 
@@ -1058,10 +1081,11 @@ SO3D_HD SeriesLaneState igso3_series_lane(float kap, float kapp, float cexp, int
 }
 // Terms the warp actually needs: the weights beyond igso3_series_live_terms(eps) are exactly 0 (ex2.approx.ftz flushes them), so
 // summing min(L, live) terms gives the bits of summing L -- and with one rotation per warp the count is warp-uniform.
+// Below 32 live terms the count is rounded up to one term per lane, but never past L: terms l >= L must not be summed.
 SO3D_HD int igso3_series_live_terms(float eps, int L);
 SO3D_HD int igso3_series_warp_terms(float eps, int L) {
   const int live = igso3_series_live_terms(eps, L);
-  return live < 32 ? 32 : live;
+  return live < 32 ? (L < 32 ? L : 32) : live;
 }
 SO3D_HD int igso3_series_lane_terms(int L) { return (L + 31) / 32; }
 SO3D_HD void igso3_series_lane_setup(float w, float eps, float* kap, float* kapp, float* cexp) {

@@ -113,7 +113,11 @@ class IsotropicGaussianSO3(Distribution):
         return ops.igso3_density(t.expand(shape).contiguous(), self.eps.expand(shape).contiguous(), mode=self.eval_mode, L=self.series_terms)
 
     def log_prob(self, rotations):
-        """distributions.py:74-77: log f_eps(angle(R)), shape (..., 1).  Differentiable w.r.t. rotations."""
+        """distributions.py:74-77: log f_eps(angle(R)), shape (..., 1).  Differentiable w.r.t. rotations, not w.r.t. eps:
+        with grad mode on and an eps that requires grad this raises instead of returning a result without that gradient."""
+        if torch.is_grad_enabled() and isinstance(self.eps, torch.Tensor) and self.eps.requires_grad:
+            raise NotImplementedError("IsotropicGaussianSO3.log_prob: the gradient w.r.t. eps is not implemented; pass eps.detach() "
+                                      "or evaluate under torch.no_grad()")
         if torch.is_grad_enabled() and rotations.requires_grad:
             return _LogProb.apply(rotations, self.eps, self.eval_mode, self.series_terms)[..., None]
         logp, _, _ = ops.igso3_logp_score(rotations, self.eps, mode=self.eval_mode, L=self.series_terms, want_score=False)

@@ -18,6 +18,7 @@ from math import log
 from typing import Iterable, Tuple
 
 import torch
+import torch.nn.functional as F
 
 from . import ops
 
@@ -238,7 +239,10 @@ def rmat_to_aa(r_mat) -> Tuple[torch.Tensor, torch.Tensor]:
     if _needs_grad(r_mat):
         skew_vec = skew2vec(_LogRmat.apply(r_mat))
         angle = skew_vec.norm(p=2, dim=-1, keepdim=True)
-        return skew_vec / angle, angle
+        # the identity gets the kernel's axis (0,0,1) (Q10); the safe denominator keeps NaN out of the backward too
+        nz = angle > 0
+        axis = torch.where(nz, skew_vec / torch.where(nz, angle, torch.ones_like(angle)), F.pad(torch.ones_like(angle), (2, 0)))
+        return axis, angle
     axis, angle = ops.rmat_to_aa(r_mat)
     return axis, angle[..., None]
 

@@ -149,63 +149,6 @@ def test_so3_scale_large_scalars(dx, cuda_device):
 
 
 # ---------------------------------------------------------------------------------------------
-# autograd functions
-# ---------------------------------------------------------------------------------------------
-def test_backward_against_reference_formulas(dx, cuda_device):
-    """Custom backward kernels vs torch autograd through a float64 restatement of the reference ops."""
-    U = dx.util
-    n = 300
-    R, _, _ = rand_rots(n, 23, 2.8)
-    G = np.random.default_rng(1).standard_normal((n, 3, 3)).astype(np.float32)
-
-    def ref_log(r):  # util.py:164-176 in float64 torch
-        a = r - r.transpose(-1, -2)
-        v = torch.stack((a[..., 2, 1], -a[..., 2, 0], a[..., 1, 0]), -1)
-        s = v.norm(dim=-1) / 2
-        c = (torch.einsum("...ii", r) - 1) / 2
-        return (torch.atan2(s, c) / (2 * s))[..., None, None] * a
-
-    r64 = torch.tensor(R, dtype=torch.float64, requires_grad=True)
-    (ref_g,) = torch.autograd.grad((ref_log(r64) * torch.tensor(G, dtype=torch.float64)).sum(), r64)
-    rd = dev(R, cuda_device).requires_grad_(True)
-    (got,) = torch.autograd.grad((U.log_rmat(rd) * dev(G, cuda_device)).sum(), rd)
-    scale = np.abs(ref_g.numpy()).max((-1, -2), keepdims=True)
-    assert np.max(np.abs(host(got) - ref_g.numpy()) / np.maximum(scale, 1.0)) < 2e-5
-
-    # so3_scale: matrix_exp(s * log R), util.py:349-361
-    s = np.random.default_rng(2).uniform(0.1, 1.5, n).astype(np.float32)
-    s64 = torch.tensor(s, dtype=torch.float64, requires_grad=True)
-    out64 = torch.matrix_exp(ref_log(r64) * s64[..., None, None])
-    ref_gr, ref_gs = torch.autograd.grad((out64 * torch.tensor(G, dtype=torch.float64)).sum(), (r64, s64))
-    sd = dev(s, cuda_device).requires_grad_(True)
-    got_r, got_s = torch.autograd.grad((U.so3_scale(rd, sd) * dev(G, cuda_device)).sum(), (rd, sd))
-    assert np.max(np.abs(host(got_s) - ref_gs.numpy())) < 2e-5 * max(1.0, np.abs(ref_gs.numpy()).max())
-    scale = np.abs(ref_gr.numpy()).max((-1, -2), keepdims=True)
-    assert np.max(np.abs(host(got_r) - ref_gr.numpy()) / np.maximum(scale, 1.0)) < 5e-5
-    # shared scalar: gradient is reduced over the batch
-    s0 = torch.tensor(0.7, device=cuda_device, requires_grad=True)
-    (g0,) = torch.autograd.grad((U.so3_scale(rd.detach(), s0) * dev(G, cuda_device)).sum(), s0)
-    s0_64 = torch.tensor(0.7, dtype=torch.float64, requires_grad=True)
-    (r0,) = torch.autograd.grad((torch.matrix_exp(ref_log(r64.detach()) * s0_64) * torch.tensor(G, dtype=torch.float64)).sum(), s0_64)
-    assert abs(g0.item() - r0.item()) < 1e-3 * max(1.0, abs(r0.item()))
-
-    # aa_to_rmat: matrix_exp(hat(axis/|axis|) * ang), util.py:195-205 (without the SVD projection)
-    axes = np.random.default_rng(3).standard_normal((n, 3)).astype(np.float32) * 2
-    ang = np.random.default_rng(4).uniform(0.01, 3.0, (n, 1)).astype(np.float32)
-    a64 = torch.tensor(axes, dtype=torch.float64, requires_grad=True)
-    an64 = torch.tensor(ang, dtype=torch.float64, requires_grad=True)
-    nrm = a64 / a64.norm(dim=-1, keepdim=True)
-    K = torch.zeros(n, 3, 3, dtype=torch.float64)
-    K = torch.stack((torch.zeros(n, dtype=torch.float64), -nrm[:, 2], nrm[:, 1], nrm[:, 2], torch.zeros(n, dtype=torch.float64), -nrm[:, 0],
-                     -nrm[:, 1], nrm[:, 0], torch.zeros(n, dtype=torch.float64)), -1).reshape(n, 3, 3)
-    ref_ga, ref_gan = torch.autograd.grad((torch.matrix_exp(K * an64[..., None]) * torch.tensor(G, dtype=torch.float64)).sum(), (a64, an64))
-    ad, and_ = dev(axes, cuda_device).requires_grad_(True), dev(ang, cuda_device).requires_grad_(True)
-    got_a, got_an = torch.autograd.grad((U.aa_to_rmat(ad, and_) * dev(G, cuda_device)).sum(), (ad, and_))
-    assert np.max(np.abs(host(got_a) - ref_ga.numpy())) < 2e-5 * max(1.0, np.abs(ref_ga.numpy()).max())
-    assert np.max(np.abs(host(got_an) - ref_gan.numpy())) < 2e-5 * max(1.0, np.abs(ref_gan.numpy()).max())
-
-
-# ---------------------------------------------------------------------------------------------
 # L1: IGSO(3)
 # ---------------------------------------------------------------------------------------------
 def eset(n, seed, kmax=4.0):
@@ -590,13 +533,20 @@ def test_two_row_engine_equals_one_row_for_the_maps(dx, cuda_device, monkeypatch
     v0 = torch.randn(n, 3, device=cuda_device, generator=g) * 0.7
     sc0 = torch.rand(n, device=cuda_device, generator=g) + 0.5
     w = torch.randn(n, 3, 3, device=cuda_device, generator=g)
+    ev = torch.rand(n, device=cuda_device, generator=g) + 0.05
+    buf = torch.empty(n * 9 + 1, device=cuda_device)
     grads = {}
     for lanes in ("1", "2"):
         monkeypatch.setenv("SO3D_ROW_LANES", lanes)
         Rr = R.clone().requires_grad_(True); vv = v0.clone().requires_grad_(True); ss = sc0.clone().requires_grad_(True)
+        ee = (v0 * 3).clone().requires_grad_(True)
+        Ru = buf[1:].view(n, 3, 3); Ru.copy_(R); Ru.requires_grad_(True)   # 4-byte aligned view: the scalar load path
         loss = (dx.util.log_rmat(Rr) * w).sum() + (dx.util.so3_scale(Rr, ss) * w).sum() + (dx.util.aa_to_rmat(vv, ss[:, None]) * w).sum()
+        loss = loss + (dx.util.exp_vec(ee) * w).sum() + (dx.util.log_rmat(Ru) * w).sum()
+        loss = loss + (dx.IsotropicGaussianSO3(ev, mode="closed").log_prob(Rr) * ss[:, None]).sum()
         loss.backward()
-        grads[lanes] = (Rr.grad.clone(), vv.grad.clone(), ss.grad.clone())
+        grads[lanes] = (Rr.grad.clone(), vv.grad.clone(), ss.grad.clone(), ee.grad.clone(), Ru.grad.clone())
+        Ru.requires_grad_(False)
     for x, y in zip(grads["1"], grads["2"]):
         assert torch.equal(x, y)
 

@@ -373,6 +373,21 @@ def test_backward_pieces(hm):
             lp = O.log_rmat(R64 + d, reference_quirks=True); lm = O.log_rmat(R64 - d, reference_quirks=True)
             num[:, i, j] = ((lp - lm) * G).sum((-1, -2)) / (2 * h)
     assert np.max(np.abs(out - num) / np.maximum(np.abs(num).max((-1, -2), keepdims=True), 1.0)) < 2e-4
+    # near pi: the tangent part vee_adj(R^T g) is the derivative of log along R exp(hat(xi)), Jr^-T(phi) vee_adj(G),
+    # to ~2^-24/sin(theta) (the reference formula's own tangent part is off by ~2^-24/sin^2(theta) on an fp32 matrix)
+    th = rng.uniform(2.6, math.pi - 1e-3, n)
+    ax = rng.standard_normal((n, 3)); ax /= np.linalg.norm(ax, axis=-1, keepdims=True)
+    Rp = f32(O.rodrigues(ax, th))
+    hm.hm_log_bwd(fp(Rp), fp(G), fp(out), ctypes.c_long(n))
+    vadj = lambda m: np.stack((m[..., 2, 1] - m[..., 1, 2], m[..., 0, 2] - m[..., 2, 0], m[..., 1, 0] - m[..., 0, 1]), -1)
+    phi = O.log_vec(Rp.astype(np.float64))
+    t = np.linalg.norm(phi, axis=-1, keepdims=True)
+    nn_, u = phi / t, vadj(G.astype(np.float64))
+    nu = np.cross(nn_, u)
+    want = u - t / 2 * nu + (1 - (t / 2) * np.sin(t) / (2 * np.sin(t / 2) ** 2)) * np.cross(nn_, nu)
+    tau = vadj(np.swapaxes(Rp.astype(np.float64), -1, -2) @ out.astype(np.float64))
+    err = np.linalg.norm(tau - want, axis=-1) / np.maximum(np.linalg.norm(want, axis=-1), 1.0)
+    assert np.all(err < 2e-5 + 8 * 2.0 ** -24 / np.sin(t[:, 0]))
     # aa_to_rmat
     axes = f32(rng.standard_normal((n, 3)) * 2); ang = f32(rng.uniform(0.01, 3.0, n))
     ga = np.empty((n, 3), np.float32); gang = np.empty(n, np.float32)
@@ -548,12 +563,14 @@ def test_series_warp_split(hm):
         assert np.all(g[om == 0] == 0)
     # short truncations (one or two terms per lane; a truncated series is only meaningful once it has converged: eps >= 0.5)
     eb = np.maximum(eps, 0.5).astype(np.float32)
-    for L in (33, 64):
+    for L in (1, 5, 33, 64):   # (below 32 terms, fewer than one per lane: no term l >= L may be summed)
         lw = np.empty(n, np.float32); gw = np.empty(n, np.float32); l1 = np.empty(n, np.float32); g1 = np.empty(n, np.float32)
         hm.hm_series_warp(fp(om), fp(eb), fp(lw), fp(gw), ctypes.c_long(n), L, 0)
         hm.hm_logf_g(fp(om), fp(eb), fp(l1), fp(g1), ctypes.c_long(n), 4, L)
         ok = om <= 4.2 * eb     # (beyond the guard both sums are rounding noise times the condition number)
         assert np.max(np.abs(np.exp(lw.astype(np.float64) - l1.astype(np.float64)) - 1)[ok]) < 8e-6, L   # (cond 14 at the guard: ~4 u cond each)
+        if L == 1:
+            assert np.all(lw == 0) and np.all(gw == 0)   # f = 1: log f = 0 and d log f / d omega = 0
     # raw sum: against the one-thread recurrence (mode series_pure)
     lw = np.empty(n, np.float32); gw = np.empty(n, np.float32); l1 = np.empty(n, np.float32); g1 = np.empty(n, np.float32)
     hm.hm_series_warp(fp(om), fp(eps), fp(lw), fp(gw), ctypes.c_long(n), 2000, 0)
