@@ -1580,6 +1580,41 @@ __global__ void __launch_bounds__(kTile) cdf_guide_kernel(const float* __restric
 // ------------------------------------------------------------------------------------------------
 // L1: sampling (distributions.py:33-51).  kShared: every sample uses one CDF row (scalar eps).
 // ------------------------------------------------------------------------------------------------
+// The two halves of SampleOp::row around the angle, for the exact sampler.  (SampleOp keeps its own inline copy: routed
+// through these helpers it compiles to different SASS.)
+// Axis and uniform of row i: explicit draws where given, else Philox(key, row_offset + i).
+__device__ __forceinline__ NoiseDraw sample_draw(const float* u_in, const float* axes_in, const PhiloxKey& key, uint64_t row_offset,
+                                                 int64_t i) {
+  NoiseDraw out;
+  if (axes_in) {
+    const float ax = axes_in[3 * i], ay = axes_in[3 * i + 1], az = axes_in[3 * i + 2];
+    const float inv = 1.0f / sqrtf(fmaf(ax, ax, fmaf(ay, ay, az * az)));  // distributions.py:36
+    out.axis = Vec3{ax * inv, ay * inv, az * inv};
+  }
+  if (!axes_in || !u_in) {
+    const NoiseDraw d = draw_axis_u(key, row_offset + (uint64_t)i);
+    if (!axes_in) out.axis = d.axis;
+    out.u = d.u;
+  }
+  if (u_in) out.u = u_in[i];
+  return out;
+}
+// mean @ exp(ang hat(axis)) (distributions.py:38-50) and the optional axis / angle outputs of row i.
+__device__ __forceinline__ void sample_finish(Vec3 axis, float ang, const float* mean, int mean_stride, float* angle_out, int64_t i,
+                                              Mat3* o9, Vec3* o3) {
+  Mat3 out = quat_to_mat_unit(quat_axis_angle(axis, ang));
+  if (mean) {
+    Mat3 m;
+    const float* mp = mean + (mean_stride ? 9 * i : 0);
+#pragma unroll
+    for (int k = 0; k < 9; ++k) m.m[k] = __ldg(mp + k);
+    out = mul_nn(m, out);
+  }
+  o9[0] = out;
+  o3[0] = axis;
+  if (angle_out) angle_out[i] = ang;
+}
+
 template <bool kShared>
 struct SampleOp {
   SO3D_OP_ARRAYS(0, 0, 1, 1)
@@ -1631,6 +1666,29 @@ struct SampleOp {
     o9[0] = out;
     o3[0] = axis;
     if (angle_out) angle_out[i] = ang;
+  }
+};
+
+// distributions.py:33-51 with the angle from the exact inverse CDF of the IGSO(3) angle law instead of the table
+// (igso3_angle_icdf, so3d_math.cuh): per-row or shared eps, nothing staged.  Compute-bound (up to 16 Newton steps of a
+// 16-node quadrature or a <= 24-term series per row), so rows run on the warp-autonomous schedule: the step count varies
+// per row, and a warp that finishes early streams its outputs without waiting for the CTA.
+struct SampleExactOp {
+  SO3D_OP_ARRAYS(0, 0, 1, 1)
+  SO3D_OP_NO_TAB
+  static constexpr bool kWarpSchedule = true;
+  const float* eps;
+  int eps_stride;
+  const float* u_in;
+  const float* axes_in;
+  PhiloxKey key;  // (seed, rng_offset), built by the launcher: the table sampler's counter layout
+  uint64_t row_offset;
+  const float* mean;
+  int mean_stride;
+  float* angle_out;
+  __device__ void row(int64_t i, const Mat3*, const Vec3*, Mat3* o9, Vec3* o3, const float*) const {
+    const NoiseDraw d = sample_draw(u_in, axes_in, key, row_offset, i);
+    sample_finish(d.axis, igso3_angle_icdf(d.u, __ldg(eps + (eps_stride ? i : 0))), mean, mean_stride, angle_out, i, o9, o3);
   }
 };
 
@@ -2868,6 +2926,21 @@ int so3d_igso3_sample_f32(const float* cdf, const uint32_t* guide, const float* 
   if (row_idx)
     return launch_sample<false>(cdf, guide, loc, rows, row_idx, 0, u, axes3, seed, rng_offset, row_offset, mean, mean_stride, R, angle, axis3, n, stream);
   return launch_sample<true>(cdf, guide, loc, rows, nullptr, row, u, axes3, seed, rng_offset, row_offset, mean, mean_stride, R, angle, axis3, n, stream);
+}
+
+int so3d_igso3_sample_exact_f32(const float* eps, int eps_stride, const float* u, const float* axes3, uint64_t seed, uint64_t rng_offset,
+                                uint64_t row_offset, const float* mean, int mean_stride, float* R, float* angle, float* axis3, int64_t n,
+                                void* stream) {
+  SO3D_REQUIRE(n >= 0, "negative n");
+  if (n == 0) return 0;
+  SO3D_REQUIRE(eps && R, "so3d_igso3_sample_exact_f32: null pointer");
+  SO3D_REQUIRE(eps_stride == 0 || eps_stride == 1, "eps_stride must be 0 or 1");
+  SO3D_REQUIRE(mean_stride == 0 || mean_stride == 1, "mean_stride must be 0 or 1");
+  SampleExactOp op;
+  op.out9[0] = R; op.out3[0] = axis3;
+  op.eps = eps; op.eps_stride = eps_stride; op.u_in = u; op.axes_in = axes3;
+  op.key = make_philox_key(seed, rng_offset); op.row_offset = row_offset; op.mean = mean; op.mean_stride = mean_stride; op.angle_out = angle;
+  return launch_rowwise_pick(op, n, stream, "so3d_igso3_sample_exact_f32");
 }
 
 int so3d_q_sample_f32(const float* x0, const int64_t* t, const float* sqrt_ac, const float* sqrt_1m_ac, int64_t T,

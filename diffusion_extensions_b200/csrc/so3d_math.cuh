@@ -1643,4 +1643,105 @@ SO3D_HD NoiseDraw draw_axis_u(uint64_t seed, uint64_t row, uint64_t offset) { re
 SO3D_HD NoiseDraw draw_axis_u(const PhiloxKey& k, uint64_t row) { return draw_from_block(philox4x32_10(k, row)); }
 SO3D_HD NoiseDraw draw_axis_u(const PhiloxRoundKeys& k, uint64_t row, uint64_t offset) { return draw_from_block(philox4x32_10(k, row, offset)); }
 
+// ------------------------------------------------------------------------------------------------
+// Exact IGSO(3) angle sampler (so3d_igso3_sample_exact_f32): w = F^{-1}(u) for the angle law
+//     p(w) = f(w) (1 - cos w) / pi  on [0, pi],   F(w) = int_0^w p,
+// found per row in registers by a safeguarded Newton iteration, with no CDF table (DESIGN.md, "Exact IGSO(3) sampler").
+// ------------------------------------------------------------------------------------------------
+constexpr float kExactSeriesEps = 0.3f;  // series antiderivative at eps >= this, Gauss-Legendre quadrature below
+constexpr float kExactXMax = 5.0f;       // eps < kExactSeriesEps: the mass beyond x = w / (2 eps) = 5 is 7.8e-11
+constexpr int kExactMaxTerms = 24;       // eps >= kExactSeriesEps: a_l < 1e-10 from l = 17 on
+constexpr int kExactIters = 16;          // Newton / bisection steps at most
+constexpr float kExactTol = 1e-6f;       // relative Newton step at which the iteration stops
+
+struct AngleCdf {
+  float F, p;  // F and dF/dz in the variable z the branch iterates in (w for the series, x = w / (2 eps) below)
+};
+
+// eps >= kExactSeriesEps.  With the density's series weights a_l = (2l+1) e^{-l(l+1) eps^2} and a_0 = 1,
+//   f(w) (1 - cos w) = sum_{l>=0} a_l [cos(l w) - cos((l+1) w)], so
+//   pi F(w) = w + sum_{l>=1} (a_l - a_{l-1}) sin(l w) / l,   pi p(w) = 1 + sum_{l>=1} (a_l - a_{l-1}) cos(l w),
+// exact on [0, pi] (F(pi) = 1).  At eps >= 0.3 the |a_l - a_{l-1}| sum to < 5, so fp32 keeps F to ~1e-7 absolute.
+// sin / cos(l w) come from the angle-addition recurrence; the sum stops once a_{l-1} < 1e-10.
+SO3D_HD AngleCdf igso3_angle_cdf_series(float w, float v) {
+  float s1, c1;
+  sincos_fast(w, &s1, &c1);
+  float sl = s1, cl = c1, F = w, p = 1.0f, a_prev = 1.0f;
+#pragma unroll 1
+  for (int l = 1; l <= kExactMaxTerms && a_prev >= 1e-10f; ++l) {
+    const float a = (float)(2 * l + 1) * expf(-(float)(l * (l + 1)) * v);
+    const float c = a - a_prev;
+    F = fmaf(c / (float)l, sl, F);
+    p = fmaf(c, cl, p);
+    const float sn = fmaf(sl, c1, cl * s1), cn = fmaf(cl, c1, -sl * s1);
+    sl = sn;
+    cl = cn;
+    a_prev = a;
+  }
+  return AngleCdf{F * (1.0f / kPi), p * (1.0f / kPi)};
+}
+
+// eps < kExactSeriesEps, in x = w / (2 eps).  The closed form without its images (they weigh < 1e-11 on w <= 10 eps < pi):
+//   dF/dx = C x sin(eps x) e^{-x^2},   C = 4 e^{eps^2/4} / (sqrt(pi) eps),   int_0^inf dF = 1 exactly,
+// integrated over [0, min(x, 5)] with 16-node Gauss-Legendre (quadrature error <= 1e-10 there for every eps < 0.3;
+// 12 nodes leave 5e-7).  As eps -> 0 this is the Maxwell law of x, i.e. w / (sqrt(2) eps) ~ chi with 3 degrees of freedom.
+SO3D_HD float igso3_angle_integrand(float x, float eps) {
+  float s, c;
+  sincos_fast(eps * x, &s, &c);
+  return x * s * expf(-x * x);
+}
+SO3D_HD AngleCdf igso3_angle_cdf_quad(float x, float eps, float C) {
+  constexpr float kNode[8] = {9.501250984e-02f, 2.816035508e-01f, 4.580167777e-01f, 6.178762444e-01f,
+                              7.554044084e-01f, 8.656312024e-01f, 9.445750231e-01f, 9.894009350e-01f};
+  constexpr float kWeight[8] = {1.894506105e-01f, 1.826034150e-01f, 1.691565194e-01f, 1.495959888e-01f,
+                                1.246289713e-01f, 9.515851168e-02f, 6.225352394e-02f, 2.715245941e-02f};
+  const float h = 0.5f * fminf(x, kExactXMax);
+  float acc = 0.0f;
+#pragma unroll
+  for (int k = 7; k >= 0; --k)
+    acc = fmaf(kWeight[k], igso3_angle_integrand(h * (1.0f - kNode[k]), eps) + igso3_angle_integrand(h * (1.0f + kNode[k]), eps), acc);
+  return AngleCdf{C * h * acc, C * igso3_angle_integrand(x, eps)};
+}
+
+// Starting point: the Maxwell quantile (the eps -> 0 law in x).  Normal quantile by Abramowitz & Stegun 26.2.23
+// (|error| < 4.5e-4), Wilson-Hilferty for chi^2_3 = 2 x^2, and in the lower tail, where Wilson-Hilferty undershoots,
+// the cubic law F ~ 4 x^3 / (3 sqrt(pi)).
+SO3D_HD float maxwell_quantile_approx(float u) {
+  const float q = fminf(u, 1.0f - u);
+  const float t = sqrtf(-2.0f * logf(q));
+  float z = t - fmaf(fmaf(0.010328f, t, 0.802853f), t, 2.515517f) / fmaf(fmaf(fmaf(0.001308f, t, 0.189269f), t, 1.432788f), t, 1.0f);
+  z = u < 0.5f ? -z : z;
+  const float h = fmaf(z, 0.27216553f, 0.92592593f);  // 1 - 2/27 + z sqrt(2/27)
+  const float xw = sqrtf(fmaxf(1.5f * h * h * h, 0.0f));
+  return fmaxf(xw, cbrtf(1.32934039f * u));  // (3 sqrt(pi) / 4) u
+}
+
+// w = F^{-1}(u) in [0, pi].  u <= 0 or eps = 0 gives 0; a NaN u or eps gives NaN.  The law depends on eps^2 only.
+// The iteration keeps a bracket [lo, hi] from the sign of F - u and replaces a Newton step that leaves it by bisection.
+SO3D_HD float igso3_angle_icdf(float u, float eps) {
+  eps = fabsf(eps);
+  if (isnan(u) || isnan(eps)) return u + eps;
+  if (u <= 0.0f || eps == 0.0f) return 0.0f;
+  const bool series = eps >= kExactSeriesEps;
+  const float v = eps * eps;
+  const float C = 4.0f * expf(0.25f * v) / (1.7724538509055159f * eps);
+  const float x0 = maxwell_quantile_approx(u);
+  float lo = 0.0f, hi = series ? kPi : kExactXMax;
+  float z = series ? fminf(2.0f * eps * x0, kPi) : fminf(x0, kExactXMax);
+#pragma unroll 1
+  for (int it = 0; it < kExactIters; ++it) {
+    const AngleCdf c = series ? igso3_angle_cdf_series(z, v) : igso3_angle_cdf_quad(z, eps, C);
+    const float r = c.F - u;
+    if (r == 0.0f) break;
+    if (r > 0.0f) hi = z;
+    else lo = z;
+    float zn = z - r / c.p;
+    if (!(zn >= lo && zn <= hi)) zn = 0.5f * (lo + hi);
+    const bool done = fabsf(zn - z) <= kExactTol * z;
+    z = zn;
+    if (done) break;
+  }
+  return series ? z : fminf(2.0f * eps * z, kPi);
+}
+
 }  // namespace so3d

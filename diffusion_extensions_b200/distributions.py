@@ -23,6 +23,11 @@ result is <= 1e-5 relative on the whole E-set), "series_pure" (the raw fp32 seri
 ``reference_quirks=True`` builds the CDF table from the reference's literal overflowing expression
 (density zeroed beyond omega > 709 eps^2/pi, SURVEY D5) so that samples match the reference at
 tiny eps too.  Quirk Q1 (column-0 gather with batched eps) is a plain bug and is not reproduced.
+``sampler`` selects how ``sample`` finds the angle: "table" (default: the reference's piecewise-linear inversion of the
+999-point trapezoid CDF above, built per distinct eps) or "exact" (the inverse CDF of the IGSO(3) angle law itself, found
+per row in registers with no table: |F(angle) - u| ~ 3e-7, and per-row eps costs 4 bytes per row instead of a 3996-byte
+table row; ``trap`` / ``table`` still build the table if read).  The quirks belong to the table, so ``sampler="exact"``
+with ``reference_quirks=True`` raises.
 """
 import torch
 from torch.distributions import Distribution, MultivariateNormal, Normal, constraints
@@ -48,7 +53,12 @@ class IsotropicGaussianSO3(Distribution):
     arg_constraints = {"eps": constraints.positive}
 
     def __init__(self, eps: torch.Tensor, mean: torch.Tensor = None, mode: str = "auto", series_terms: int = 2000,
-                 reference_quirks: bool = False):
+                 reference_quirks: bool = False, sampler: str = "table"):
+        if sampler not in ("table", "exact"):
+            raise ValueError(f"sampler must be 'table' or 'exact' (got {sampler!r})")
+        if sampler == "exact" and reference_quirks:
+            raise ValueError("sampler='exact' draws from the IGSO(3) law itself; reference_quirks only shape the CDF table of "
+                             "sampler='table'")
         if not isinstance(eps, torch.Tensor):
             raise TypeError("eps must be a torch.Tensor on a CUDA device")
         if not eps.is_cuda:
@@ -58,6 +68,7 @@ class IsotropicGaussianSO3(Distribution):
         self.eval_mode = mode
         self.series_terms = int(series_terms)
         self.reference_quirks = bool(reference_quirks)
+        self.sampler = sampler
         self._table = None  # (E_flat, 999), built on first use
         super().__init__(batch_shape=self.eps.shape, validate_args=False)
 
@@ -96,6 +107,9 @@ class IsotropicGaussianSO3(Distribution):
             # a batched mean broadcasts against the noise like the reference's `self._mean @ rotations`
             # (distributions.py:50; e.g. IGSO3xR3(eps=sigma[0], mean=model_mean).sample() at diffusion.py:482 -> (B,3,3))
             shape = tuple(torch.broadcast_shapes(shape, self._mean.shape[:-2]))
+        if self.sampler == "exact":
+            eps = self.eps if self.eps.numel() == 1 else self.eps.expand(shape)
+            return ops.igso3_sample_exact(eps, shape, u=u, axes=axes, row_offset=row_offset, mean=self._mean, want_angle=return_angle)
         if self.eps.dim() == 0:
             row_idx, row = None, 0
         else:

@@ -459,6 +459,47 @@ def igso3_sample(cdf, shape, row_idx=None, row=0, u=None, axes=None, seed=None, 
     return outs[0] if len(outs) == 1 else tuple(outs)
 
 
+def igso3_sample_exact(eps, shape, u=None, axes=None, seed=None, rng_offset=None, row_offset=0, mean=None,
+                       want_angle=False, want_axis=False):
+    """Draw rotations of batch shape `shape` from IGSO(3)(eps) with the angle from the exact inverse CDF of the angle law
+    (no CDF table: per-row eps costs one float per row).  eps: a scalar / one-element tensor, or a tensor that broadcasts
+    to `shape` (one eps per sample).  u / axes / seed / rng_offset / row_offset / mean as in `igso3_sample`, with the same
+    Philox counter layout: at the same (seed, rng_offset, row_offset) both samplers draw the same (u, axis).
+    -> R (*shape,3,3)[, angle (*shape)][, axis (*shape,3)]"""
+    shape = tuple(shape)
+    if isinstance(eps, torch.Tensor):
+        dev = eps.device
+    else:
+        dev = torch.device("cuda", torch.cuda.current_device())
+    n = 1
+    for d in shape:
+        n *= int(d)
+    eps_t, eps_stride = _per_row(eps, shape, dev, "eps")
+    if u is not None:
+        u = check_f32(u, "u").expand(shape).contiguous()
+    if axes is not None:
+        axes = check_f32(axes, "axes", (3,)).expand(*shape, 3).contiguous()
+    if seed is None or rng_offset is None:
+        seed, rng_offset = rng.next()
+    mean_stride = 0
+    if mean is not None:
+        mean = check_f32(mean, "mean", (3, 3))
+        if mean.numel() != 9:
+            mean = mean.expand(*shape, 3, 3).contiguous()
+            mean_stride = 1
+    R = torch.empty(*shape, 3, 3, dtype=torch.float32, device=dev)
+    angle = torch.empty(shape, dtype=torch.float32, device=dev) if want_angle else None
+    axis_out = torch.empty(*shape, 3, dtype=torch.float32, device=dev) if want_axis else None
+    call("so3d_igso3_sample_exact_f32", ptr(eps_t), eps_stride, ptr(u), ptr(axes), seed, rng_offset, int(row_offset), ptr(mean),
+         mean_stride, ptr(R), ptr(angle), ptr(axis_out), n, device=dev)
+    outs = [R]
+    if want_angle:
+        outs.append(angle)
+    if want_axis:
+        outs.append(axis_out)
+    return outs[0] if len(outs) == 1 else tuple(outs)
+
+
 # ---------------------------------------------------------------------------------------------
 # SE(3) arm: fused forward noising / reverse step on (rotation, translation) pairs (diffusion.py:432-573)
 # ---------------------------------------------------------------------------------------------

@@ -128,6 +128,14 @@ int so3d_igso3_sample_f32(const float* cdf, const uint32_t* guide, const float* 
                           const float* u, const float* axes3, uint64_t seed, uint64_t rng_offset,
                           uint64_t row_offset, const float* mean, int mean_stride, float* R, float* angle,
                           float* axis3, int64_t n, void* stream);
+/* The same draw with no table: the angle is the exact inverse CDF of the IGSO(3) angle law
+ * p(w) = f_eps(w) (1 - cos w) / pi on [0, pi], found per row (|F(angle) - u| ~ 3e-7 for eps in [1e-3, 4]).
+ *   eps: eps_stride 0 (one shared eps) or 1 (eps[n], one per row).  u = 0 gives angle 0; a NaN eps a NaN angle.
+ *   u / axes3 / seed / rng_offset / row_offset / mean / outputs as in so3d_igso3_sample_f32, with the same Philox
+ *   counter layout, so at the same seed both samplers see the same (u, axis). */
+int so3d_igso3_sample_exact_f32(const float* eps, int eps_stride, const float* u, const float* axes3, uint64_t seed,
+                                uint64_t rng_offset, uint64_t row_offset, const float* mean, int mean_stride, float* R,
+                                float* angle, float* axis3, int64_t n, void* stream);
 
 /* ---- L2: diffusion.py SO3Diffusion ---------------------------------------------------------- */
 /* diffusion.py:339-346 q_sample + :348-355 p_losses target, fused:
