@@ -275,13 +275,16 @@ template <class L>
 SO3D_HD AxisAngleL<L> axis_angle_fast_l(const Mat3L<L>& r) {
   using M = typename MaskOf<L>::type;
   const L zero = bc<L>(0.f);
-  const L vx = sub(r.m[7], r.m[5]), vy = sub(r.m[2], r.m[6]), vz = sub(r.m[3], r.m[1]);
+  const L ux = sub(r.m[7], r.m[5]), uy = sub(r.m[2], r.m[6]), uz = sub(r.m[3], r.m[1]);
+  const M tiny = lt(fma(ux, ux, fma(uy, uy, mul(uz, uz))), bc<L>(kFltMin));
+  const L k = sel(tiny, bc<L>(kTinyUp), bc<L>(1.0f));
+  const L vx = mul(ux, k), vy = mul(uy, k), vz = mul(uz, k);
   const L n2 = fma(vx, vx, fma(vy, vy, mul(vz, vz)));
-  const M pos = gt(n2, zero);
+  const M pos = ge(n2, bc<L>(kFltMin));
   const L rs = sel(pos, vrsqrt(n2), zero);
   const L c = mulc(0.5f, add(add(add(r.m[0], r.m[4]), r.m[8]), bc<L>(-1.0f)));
   AxisAngleL<L> o;
-  o.theta = atan2_pos_l(mul(mulc(0.5f, n2), rs), c);
+  o.theta = atan2_pos_l(mul(mul(sel(tiny, bc<L>(0.5f * kTinyDown), bc<L>(0.5f)), n2), rs), c);
   const L d0 = sub(r.m[0], c), d1 = sub(r.m[4], c), d2 = sub(r.m[8], c);
   const L s01 = mulc(0.5f, add(r.m[1], r.m[3])), s02 = mulc(0.5f, add(r.m[2], r.m[6])), s12 = mulc(0.5f, add(r.m[5], r.m[7]));
   const M p0 = mand(ge(d0, d1), ge(d0, d2));
@@ -301,12 +304,15 @@ template <class L>
 SO3D_HD void quat_axis_halfangle_l(const QuatL<L>& q, Vec3L<L>* n, L* half) {
   using M = typename MaskOf<L>::type;
   const L zero = bc<L>(0.f);
-  const L v2 = fma(q.x, q.x, fma(q.y, q.y, mul(q.z, q.z)));
-  const M pos = gt(v2, zero);
+  const M tiny = lt(fma(q.x, q.x, fma(q.y, q.y, mul(q.z, q.z))), bc<L>(kFltMin));
+  const L sc = sel(tiny, bc<L>(kTinyUp), bc<L>(1.0f));
+  const L x = mul(q.x, sc), y = mul(q.y, sc), z = mul(q.z, sc);
+  const L v2 = fma(x, x, fma(y, y, mul(z, z)));
+  const M pos = ge(v2, bc<L>(kFltMin));
   const L rs = sel(pos, vrsqrt(v2), zero);
-  *half = atan2_pos_l(mul(v2, rs), vabs(q.w));
+  *half = atan2_pos_l(mul(mul(sel(tiny, bc<L>(kTinyDown), bc<L>(1.0f)), v2), rs), vabs(q.w));
   const L k = sel(lt(q.w, zero), neg(rs), rs);
-  *n = Vec3L<L>{mul(q.x, k), mul(q.y, k), sel(pos, mul(q.z, k), bc<L>(1.0f))};
+  *n = Vec3L<L>{mul(x, k), mul(y, k), sel(pos, mul(z, k), bc<L>(1.0f))};
 }
 
 // ---- the reverse step's posterior mean on quaternions (p_mean_quat / p_mean_quat_nopred) ---------------------------------

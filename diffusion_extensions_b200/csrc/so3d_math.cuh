@@ -425,17 +425,29 @@ SO3D_HD Mat3 quat_to_mat_unit(const Quat& q0) {
 // Axis and angle of a rotation matrix, branch-free: same definition as axis_angle() above (theta = atan2(|v|/2,
 // (tr-1)/2); axis from the skew part, or for (tr-1)/2 < kNearPiCos from the best-conditioned column of the
 // symmetric part (R + R^T)/2 - c I = (1 - c) n n^T, sign fixed by the skew part), selects instead of branches.
+//
+// MUFU.RSQ (rsqrt.approx.ftz) flushes a subnormal input to zero and returns +inf, which made |v|^2 below FLT_MIN
+// (theta below ~5e-20) come out as theta = pi/2 with an inf / NaN axis.  Such a skew part is scaled by 2^64 first
+// (exact), so the axis and the angle keep full relative precision down to theta ~ 1e-38; below that the row is read as
+// the identity.  For |v|^2 >= FLT_MIN the scale is 1 and every bit is what it was without it.
+constexpr float kFltMin = 1.17549435e-38f;  // FLT_MIN = 2^-126
+constexpr float kTinyUp = 18446744073709551616.0f;    // 2^64
+constexpr float kTinyDown = 5.42101086242752217e-20f;  // 2^-64
 struct AxisAngleF {
   Vec3 axis;
   float theta;
 };
 SO3D_HD AxisAngleF axis_angle_fast(const Mat3& r) {
-  const float vx = r.m[7] - r.m[5], vy = r.m[2] - r.m[6], vz = r.m[3] - r.m[1];
+  const float ux = r.m[7] - r.m[5], uy = r.m[2] - r.m[6], uz = r.m[3] - r.m[1];
+  const bool tiny = fmaf(ux, ux, fmaf(uy, uy, uz * uz)) < kFltMin;
+  const float k = fsel(tiny, kTinyUp, 1.0f);
+  const float vx = ux * k, vy = uy * k, vz = uz * k;
   const float n2 = fmaf(vx, vx, fmaf(vy, vy, vz * vz));
-  const float rs = fsel(n2 > 0.f, rsqrt_approx(n2), 0.f);
+  const bool pos = n2 >= kFltMin;
+  const float rs = fsel(pos, rsqrt_approx(n2), 0.f);
   const float c = 0.5f * (r.m[0] + r.m[4] + r.m[8] - 1.0f);
   AxisAngleF o;
-  o.theta = atan2_pos(0.5f * n2 * rs, c);
+  o.theta = atan2_pos(fsel(tiny, 0.5f * kTinyDown, 0.5f) * n2 * rs, c);
   // symmetric-part candidate: column j of S - c I with the largest diagonal
   const float d0 = r.m[0] - c, d1 = r.m[4] - c, d2 = r.m[8] - c;
   const float s01 = 0.5f * (r.m[1] + r.m[3]), s02 = 0.5f * (r.m[2] + r.m[6]), s12 = 0.5f * (r.m[5] + r.m[7]);
@@ -447,10 +459,9 @@ SO3D_HD AxisAngleF axis_angle_fast(const Mat3& r) {
   const float cn = rsqrt_approx(fmaxf(fmaf(cx, cx, fmaf(cy, cy, cz * cz)), 1e-30f));
   const float sg = fsel(fmaf(cx, vx, fmaf(cy, vy, cz * vz)) < 0.f, -cn, cn);
   const bool near_pi = c < kNearPiCos;
-  const bool ident = !(n2 > 0.f);
   o.axis.x = fsel(near_pi, cx * sg, vx * rs);
   o.axis.y = fsel(near_pi, cy * sg, vy * rs);
-  o.axis.z = fsel(near_pi, cz * sg, fsel(ident, 1.0f, vz * rs));
+  o.axis.z = fsel(near_pi, cz * sg, fsel(pos, vz * rs, 1.0f));
   return o;
 }
 
@@ -465,13 +476,18 @@ SO3D_HD Mat3 scale_rot_fast(const Mat3& r, float s) {  // util.py:349-361: rotat
   return quat_to_mat_unit(quat_axis_angle(a.axis, s * a.theta));
 }
 
-// half-angle in [0, pi/2] and unit axis of a (near-)unit quaternion, with q and -q identified
+// half-angle in [0, pi/2] and unit axis of a (near-)unit quaternion, with q and -q identified (a vector part whose
+// square is below FLT_MIN is scaled by 2^64 first, as in axis_angle_fast)
 SO3D_HD void quat_axis_halfangle(const Quat& q, Vec3* n, float* half) {
-  const float v2 = fmaf(q.x, q.x, fmaf(q.y, q.y, q.z * q.z));
-  const float rs = fsel(v2 > 0.f, rsqrt_approx(v2), 0.f);
-  *half = atan2_pos(v2 * rs, fabsf(q.w));
+  const bool tiny = fmaf(q.x, q.x, fmaf(q.y, q.y, q.z * q.z)) < kFltMin;
+  const float sc = fsel(tiny, kTinyUp, 1.0f);
+  const float x = q.x * sc, y = q.y * sc, z = q.z * sc;
+  const float v2 = fmaf(x, x, fmaf(y, y, z * z));
+  const bool pos = v2 >= kFltMin;
+  const float rs = fsel(pos, rsqrt_approx(v2), 0.f);
+  *half = atan2_pos(fsel(tiny, kTinyDown, 1.0f) * v2 * rs, fabsf(q.w));
   const float k = fsel(q.w < 0.f, -rs, rs);
-  *n = Vec3{q.x * k, q.y * k, fsel(v2 > 0.f, q.z * k, 1.0f)};
+  *n = Vec3{x * k, y * k, fsel(pos, z * k, 1.0f)};
 }
 
 // Kernel values on SO(3) for a pair of unit quaternions a, b (real part first), util.py:128-150:

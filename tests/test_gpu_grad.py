@@ -17,10 +17,10 @@ import pytest
 import torch
 
 from oracle import so3_oracle as O
+from tests.strata import Report, THETA_STRATA, U24, angle_of, pi_amp, rot_stratum, unit_axes
 
 pytestmark = pytest.mark.gpu
 
-U24 = 2.0 ** -24
 F64 = torch.float64
 
 
@@ -84,64 +84,6 @@ def tangent64(f, R):
 
 def row_max(a):
     return np.abs(a).reshape(a.shape[0], -1).max(-1)
-
-
-class Report:
-    """Per-stratum maximum of err / tol; the test fails if any stratum exceeds 1 and names it."""
-
-    def __init__(self, title):
-        self.title, self.rows = title, []
-
-    def add(self, stratum, what, err, tol):
-        err, tol = np.broadcast_to(np.asarray(err, np.float64), np.shape(tol) or np.shape(err)), np.asarray(tol, np.float64)
-        ratio = err / tol
-        ratio = np.where(np.isnan(ratio), np.inf, ratio)
-        self.rows.append((stratum, what, float(np.max(err, initial=0.0)), float(np.max(ratio, initial=0.0))))
-
-    def check(self):
-        print(f"\n{self.title}")
-        for st, what, e, r in self.rows:
-            print(f"  {st:24s} {what:22s} max err {e:9.2e}   max err/tol {r:6.3f}")
-        bad = [(st, what, e, r) for st, what, e, r in self.rows if not r <= 1.0]
-        assert not bad, f"{self.title}: over tolerance in {bad}"
-
-
-def unit_axes(rng, n):
-    ax = rng.standard_normal((n, 3))
-    return ax / np.linalg.norm(ax, axis=-1, keepdims=True)
-
-
-THETA_STRATA = [
-    ("theta=0", 0.0, 0.0), ("[1e-7,1e-4]", 1e-7, 1e-4), ("s=1e-4+-1%", 0.99e-4, 1.01e-4), ("[1e-4,1e-2]", 1e-4, 1e-2),
-    ("[1e-2,2.8]", 1e-2, 2.8), ("[2.8,3.0]", 2.8, 3.0), ("[3.0,3.1]", 3.0, 3.1), ("[3.1,pi-1e-3]", 3.1, math.pi - 1e-3),
-    ("theta=pi", math.pi, math.pi),
-]
-
-
-def rot_stratum(rng, n, lo, hi):
-    """fp32 rotations (Rodrigues in fp64, then rounded) with angles in [lo, hi] (log-uniform below 1e-2)."""
-    if lo == hi:
-        th = np.full(n, lo)
-    elif hi <= 1e-2:
-        th = np.exp(rng.uniform(math.log(lo), math.log(hi), n))
-    else:
-        th = rng.uniform(lo, hi, n)
-    R = O.rodrigues(unit_axes(rng, n), th).astype(np.float32)
-    if lo == 0.0:
-        R[:] = np.eye(3, dtype=np.float32)
-    return R
-
-
-def pi_amp(th):
-    """1/sin(theta) above pi/2, 1 below.  Near pi an fp32 matrix holds its axis only to ~2^-24/sin(theta), which bounds
-    every gradient taken through log there; near 0 the problem is well conditioned and gets no allowance."""
-    th = np.asarray(th, np.float64)
-    return np.where(th > math.pi / 2, 1.0 / np.sin(np.minimum(th, math.pi - 1e-300)), 1.0)
-
-
-def angle_of(R):
-    """angle of the fp32 matrix (fp64 evaluation)."""
-    return O.rmat_to_aa(R.astype(np.float64))[1][:, 0]
 
 
 # ---------------------------------------------------------------------------------------------
