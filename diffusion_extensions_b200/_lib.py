@@ -40,6 +40,7 @@ SIGNATURES = {
     "so3d_igso3_cdf_table_f32": [_c_f, _i64, _c_f, _c_f, _c_f, _int, _c_f],
     "so3d_igso3_sample_f32": [_c_f, _c_f, _c_f, _i64, _c_f, _i64, _c_f, _c_f, _u64, _u64, _u64, _c_f, _int, _c_f, _c_f, _c_f, _i64, _c_f],
     "so3d_igso3_sample_exact_f32": [_c_f, _int, _c_f, _c_f, _u64, _u64, _u64, _c_f, _int, _c_f, _c_f, _c_f, _i64, _c_f],
+    "so3d_igso3_rsample_bwd_f32": [_c_f, _int, _c_f, _c_f, _c_f, _int, _c_f, _c_f, _u64, _u64, _u64, _c_f, _c_f, _i64, _c_f],
     "so3d_q_sample_f32": [_c_f, _c_f, _c_f, _c_f, _i64, _c_f, _c_f, _c_f, _u64, _u64, _u64, _c_f, _c_f, _c_f, _c_f, _i64, _c_f],
     "so3d_q_sample_given_f32": [_c_f, _c_f, _c_f, _i64, _c_f, _c_f, _i64, _c_f],
     "so3d_p_sample_f32": [_c_f, _c_f, _c_f, _int, _c_f, _c_f, _c_f, _c_f, _i64, _c_f, _c_f, _c_f, _u64, _u64, _u64, _c_f, _c_f, _i64, _c_f],

@@ -1692,6 +1692,50 @@ struct SampleExactOp {
   }
 };
 
+// Backward of the reparameterised exact draw R = mean N, N = exp(w hat(a)), w = F^{-1}(u; eps) at fixed (u, a)
+// (IsotropicGaussianSO3.rsample): N is rebuilt from the sampler's axis and angle exactly as SampleExactOp forms it, then
+//   G_N = mean^T G,   g_w = <G_N, hat(a) N> = dL/dw,   g_eps = g_w dw/deps (igso3_angle_deps, so3d_math.cuh),   g_mean = G N^T.
+// dw/deps is one evaluation of the angle score at the known w, no iteration.  At eps = 0 the angle is 0 for every u and the
+// derivative is the eps -> 0+ limit 2 x0(u), so those rows (only those) re-derive u: the given u, else the sampler's Philox
+// draw at the same (seed, rng_offset, row_offset).  The per-row cost varies with eps (closed form, series above eps = 1,
+// the inversion at eps = 0), so rows run on the warp-autonomous schedule like the sampler.
+struct RsampleBwdOp {
+  SO3D_OP_ARRAYS(1, 1, 1, 0)
+  SO3D_OP_NO_TAB
+  static constexpr bool kWarpSchedule = true;
+  const float* eps;
+  int eps_stride;
+  const float* angle;
+  const float* mean;
+  int mean_stride;
+  const float* u_in;
+  PhiloxKey key;
+  uint64_t row_offset;
+  float* g_eps;
+  __device__ void row(int64_t i, const Mat3* a9, const Vec3* a3, Mat3* o9, Vec3*, const float*) const {
+    const float e = __ldg(eps + (eps_stride ? i : 0));
+    const float w = __ldg(angle + i);
+    const Mat3 nrot = quat_to_mat_unit(quat_axis_angle(a3[0], w));
+    Mat3 gn = a9[0];
+    if (mean) {
+      Mat3 m;
+      const float* mp = mean + (mean_stride ? 9 * i : 0);
+#pragma unroll
+      for (int k = 0; k < 9; ++k) m.m[k] = __ldg(mp + k);
+      gn = mul_tn(m, gn);
+    }
+    const Mat3 dn = mul_nn(hat(a3[0]), nrot);
+    float gw = 0.0f;
+#pragma unroll
+    for (int k = 0; k < 9; ++k) gw = fmaf(gn.m[k], dn.m[k], gw);
+    float d;
+    if (e == 0.0f) d = igso3_angle_deps_eps0(u_in ? __ldg(u_in + i) : draw_axis_u(key, row_offset + (uint64_t)i).u);
+    else d = igso3_angle_deps(w, e);
+    g_eps[i] = gw * d;
+    o9[0] = mul_nt(a9[0], nrot);
+  }
+};
+
 // distributions.py:113-127 Bingham.rsample: unit quaternion = normalise(L z), z ~ N(0, I4), L = scale_tril of the
 // covariance; fused with util.py:222-252 quat_to_rmat (bingham_train.py:88-90 feeds the samples straight into it).
 struct BinghamOp {
@@ -2941,6 +2985,21 @@ int so3d_igso3_sample_exact_f32(const float* eps, int eps_stride, const float* u
   op.eps = eps; op.eps_stride = eps_stride; op.u_in = u; op.axes_in = axes3;
   op.key = make_philox_key(seed, rng_offset); op.row_offset = row_offset; op.mean = mean; op.mean_stride = mean_stride; op.angle_out = angle;
   return launch_rowwise_pick(op, n, stream, "so3d_igso3_sample_exact_f32");
+}
+
+int so3d_igso3_rsample_bwd_f32(const float* eps, int eps_stride, const float* angle, const float* axis3, const float* mean,
+                               int mean_stride, const float* G9, const float* u, uint64_t seed, uint64_t rng_offset,
+                               uint64_t row_offset, float* g_eps, float* g_mean9, int64_t n, void* stream) {
+  SO3D_REQUIRE(n >= 0, "negative n");
+  if (n == 0) return 0;
+  SO3D_REQUIRE(eps && angle && axis3 && G9 && g_eps, "so3d_igso3_rsample_bwd_f32: null pointer");
+  SO3D_REQUIRE(eps_stride == 0 || eps_stride == 1, "eps_stride must be 0 or 1");
+  SO3D_REQUIRE(mean_stride == 0 || mean_stride == 1, "mean_stride must be 0 or 1");
+  RsampleBwdOp op;
+  op.in9[0] = G9; op.in3[0] = axis3; op.out9[0] = g_mean9;
+  op.eps = eps; op.eps_stride = eps_stride; op.angle = angle; op.mean = mean; op.mean_stride = mean_stride;
+  op.u_in = u; op.key = make_philox_key(seed, rng_offset); op.row_offset = row_offset; op.g_eps = g_eps;
+  return launch_rowwise_pick(op, n, stream, "so3d_igso3_rsample_bwd_f32");
 }
 
 int so3d_q_sample_f32(const float* x0, const int64_t* t, const float* sqrt_ac, const float* sqrt_1m_ac, int64_t T,

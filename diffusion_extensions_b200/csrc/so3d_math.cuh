@@ -1760,4 +1760,52 @@ SO3D_HD float igso3_angle_icdf(float u, float eps) {
   return series ? z : fminf(2.0f * eps * z, kPi);
 }
 
+// ------------------------------------------------------------------------------------------------
+// Pathwise derivative of the exact sampler's angle (so3d_igso3_rsample_bwd_f32): dw/deps of w = F^{-1}(u; eps) at fixed u
+// (DESIGN.md, "Reparameterised IGSO(3) sampling").  Implicit differentiation gives dw/deps = -(dF/deps)(w) / p(w).  The
+// density solves the heat equation on SO(3), df/d(eps^2) = f'' + cot(w/2) f' = (sin^2(w/2) f')' / sin^2(w/2), and
+// p = (2/pi) sin^2(w/2) f, so
+//     dF/d(eps^2) = (2/pi) int_0^w (sin^2(t/2) f'(t))' dt = (2/pi) sin^2(w/2) f'(w)   and   dw/deps = -2 eps f'(w) / f(w):
+// the pathwise derivative is -2 eps times the angle score d log f / dw, one evaluation at the known w.  Every image term of
+// the closed form solves the heat equation by itself, so this holds for the image-free law of the quadrature regime too.
+//   eps <  kExactSeriesEps (the sampler's quadrature regime: image-free law, log f = log x - x^2 - log sin(w/2) + const in
+//          x = w / (2 eps)):  dw/deps = 2x - 2 eps phi(w),  phi = 1/w - cot(w/2)/2 = w/12 + w^3/720 + ...;  2 eps phi is at
+//          most 2 % of 2x, so nothing cancels, and w = 0 gives 0.
+//   eps >= kExactSeriesEps (the series regime): -2 eps g with g from the density's `auto` evaluator (igso3_logf_g_t<kAuto>:
+//          the 3-image closed form up to eps = 1, the series above).  The series of F and p would not do here: in the upper
+//          tail at eps near 0.3 their terms are 10^7 times the density, and f' / f would keep no digit.
+// Special values follow the sampler: NaN eps gives NaN; the law depends on eps^2, so the result is sign(eps) dw/d|eps|.
+constexpr float kDepsPhiTaylorW = 0.5f;  // phi(w) by its Taylor series below this (4 terms: <= 2e-9 relative)
+
+SO3D_HD float igso3_angle_phi(float w) {
+  if (w < kDepsPhiTaylorW) {
+    const float w2 = w * w;
+    return w * fmaf(w2, fmaf(w2, fmaf(w2, 8.2671958e-7f, 3.3068783e-5f), 1.3888889e-3f), 8.3333333e-2f);
+  }
+  float sh, ch;
+  sincos_fast(0.5f * w, &sh, &ch);
+  return 1.0f / w - 0.5f * ch / sh;
+}
+
+SO3D_HD float igso3_angle_deps(float w, float eps) {
+  const float e = fabsf(eps);
+  float d;
+  if (isnan(e)) {
+    d = e;
+  } else if (e < kExactSeriesEps) {
+    const float x = w / (2.0f * e);
+    d = fmaf(-2.0f * e, igso3_angle_phi(w), 2.0f * x);
+  } else {
+    float lf, g;
+    igso3_logf_g_t<kAuto>(w, e, kExactMaxTerms, &lf, &g);
+    d = -2.0f * e * g;
+  }
+  return eps < 0.0f ? -d : d;
+}
+
+// eps = 0: the sampler returns w = 0 whatever u is, so the derivative comes from u.  As eps -> 0+, w = 2 eps x with x -> x0(u),
+// the Maxwell quantile, so dw/deps -> 2 x0(u).  x0 is the sampler's own quadrature-regime inversion at eps = 2^-64 (where
+// C sin(eps x) = (4/sqrt(pi)) x to fp32 and 2 eps x is exact): 2 x0 = 2^64 w.
+SO3D_HD float igso3_angle_deps_eps0(float u) { return igso3_angle_icdf(u, kTinyDown) * kTinyUp; }
+
 }  // namespace so3d

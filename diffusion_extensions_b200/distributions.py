@@ -28,8 +28,12 @@ tiny eps too.  Quirk Q1 (column-0 gather with batched eps) is a plain bug and is
 per row in registers with no table: |F(angle) - u| ~ 3e-7, and per-row eps costs 4 bytes per row instead of a 3996-byte
 table row; ``trap`` / ``table`` still build the table if read).  The quirks belong to the table, so ``sampler="exact"``
 with ``reference_quirks=True`` raises.
+``rsample`` is the reparameterised draw: always the exact inverse CDF (whatever ``sampler`` says), differentiable w.r.t. eps
+and the mean through one backward kernel.  At fixed (u, axis) the angle's derivative is dw/deps = -2 eps d log f / dw (the
+heat equation turns the implicit derivative -(dF/deps)/p into the angle score), evaluated at the sampled angle.
 """
 import torch
+from torch.autograd.function import once_differentiable
 from torch.distributions import Distribution, MultivariateNormal, Normal, constraints
 
 from . import ops
@@ -49,8 +53,37 @@ class _LogProb(torch.autograd.Function):
         return ops.igso3_logp_bwd(rotations, dlogf, grad.contiguous()), None, None, None
 
 
+class _RSample(torch.autograd.Function):
+    """R = mean exp(w hat(a)), w = F^{-1}(u; eps) by the exact sampler; u and a are constants of the draw."""
+
+    @staticmethod
+    def forward(ctx, eps, mean, eps_rows, shape, u, axes, row_offset):
+        seed, rng_offset = ops.rng.next()
+        R, angle, axis = ops.igso3_sample_exact(eps_rows, shape, u=u, axes=axes, seed=seed, rng_offset=rng_offset,
+                                                row_offset=row_offset, mean=mean, want_angle=True, want_axis=True)
+        ctx.save_for_backward(eps_rows, mean, angle, axis, u)
+        ctx.draw = (seed, rng_offset, row_offset)
+        ctx.shapes = (eps.shape, None if mean is None else mean.shape)
+        return R
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad):
+        eps_rows, mean, angle, axis, u = ctx.saved_tensors
+        seed, rng_offset, row_offset = ctx.draw
+        eps_shape, mean_shape = ctx.shapes
+        want_mean = mean is not None and ctx.needs_input_grad[1]
+        g_eps, g_mean = ops.igso3_rsample_bwd(eps_rows, angle, axis, grad, u=u, seed=seed, rng_offset=rng_offset,
+                                              row_offset=row_offset, mean=mean, want_mean_grad=want_mean)
+        g_eps = g_eps.sum().reshape(eps_shape) if eps_rows.numel() == 1 else g_eps.sum_to_size(eps_shape)
+        if want_mean:
+            g_mean = g_mean.reshape(-1, 9).sum(0).reshape(mean_shape) if mean.numel() == 9 else g_mean.sum_to_size(mean_shape)
+        return g_eps, g_mean, None, None, None, None, None
+
+
 class IsotropicGaussianSO3(Distribution):
     arg_constraints = {"eps": constraints.positive}
+    has_rsample = True
 
     def __init__(self, eps: torch.Tensor, mean: torch.Tensor = None, mode: str = "auto", series_terms: int = 2000,
                  reference_quirks: bool = False, sampler: str = "table"):
@@ -118,6 +151,25 @@ class IsotropicGaussianSO3(Distribution):
         return ops.igso3_sample(self.table, shape, row_idx=row_idx, row=row, u=u, axes=axes, row_offset=row_offset,
                                 mean=self._mean, want_angle=return_angle)
 
+    def rsample(self, sample_shape=torch.Size(), *, u=None, axes=None, row_offset=0):
+        """Reparameterised draw: rotations of shape (*sample_shape, *eps.shape, 3, 3) (broadcast against a batched mean, as in
+        ``sample``), differentiable w.r.t. eps and the mean.  The angle always comes from the exact inverse CDF of the IGSO(3)
+        law (with ``sampler="exact"`` the values are ``sample``'s, bit for bit, at the same seed).  u / axes are constants of
+        the draw (no gradient flows to them).  The gradient w.r.t. eps is sign(eps) dw/d|eps|; at eps = 0 it is the eps -> 0+
+        limit 2 x0(u), x0 the Maxwell quantile.  Once differentiable."""
+        if self.reference_quirks:
+            raise ValueError("rsample draws from the IGSO(3) law itself through the exact inverse CDF; reference_quirks only shape "
+                             "the CDF table of sampler='table'")
+        shape = tuple(sample_shape) + tuple(self.eps.shape)
+        if self._mean is not None and self._mean.dim() > 2:
+            shape = tuple(torch.broadcast_shapes(shape, self._mean.shape[:-2]))
+        eps_rows = self.eps.detach()
+        if eps_rows.numel() != 1:
+            eps_rows = eps_rows.expand(shape)
+        u = None if u is None else u.detach()
+        axes = None if axes is None else axes.detach()
+        return _RSample.apply(self.eps, self._mean, eps_rows, shape, u, axes, row_offset)
+
     # -- density (distributions.py:53-72) --------------------------------------------------------
     def _eps_ft(self, t: torch.Tensor) -> torch.Tensor:
         t = t.to(device=self.eps.device, dtype=torch.float32)
@@ -170,9 +222,10 @@ class IsotropicGaussianSO3(Distribution):
 
 class IGSO3xR3(Distribution):
     """distributions.py:84-110: product of IGSO3(eps) on the rotation and N(shift, (eps * shift_scale)^2 I) on the
-    translation of an SE(3) element (`AffineT`).  `sample` draws both halves on the device."""
+    translation of an SE(3) element (`AffineT`).  `sample` draws both halves on the device; `rsample` too, differentiably."""
 
     arg_constraints = {"eps": constraints.positive}
+    has_rsample = True
 
     def __init__(self, eps: torch.Tensor, mean: AffineT = None, shift_scale=1.0, mode: str = "auto"):
         self.eps = eps
@@ -190,6 +243,13 @@ class IGSO3xR3(Distribution):
     def sample(self, sample_shape=torch.Size()):
         rot = self.igso3.sample(sample_shape)
         shift = self.r3.sample(sample_shape)
+        return AffineT(rot, shift)
+
+    def rsample(self, sample_shape=torch.Size()):
+        """Reparameterised draw, differentiable w.r.t. eps and the mean: the rotation from ``IsotropicGaussianSO3.rsample``
+        (exact inverse CDF), the shift from ``Normal.rsample``."""
+        rot = self.igso3.rsample(sample_shape)
+        shift = self.r3.rsample(sample_shape)
         return AffineT(rot, shift)
 
     def log_prob(self, value):

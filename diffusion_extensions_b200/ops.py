@@ -500,6 +500,36 @@ def igso3_sample_exact(eps, shape, u=None, axes=None, seed=None, rng_offset=None
     return outs[0] if len(outs) == 1 else tuple(outs)
 
 
+def igso3_rsample_bwd(eps, angle, axis, G, u=None, seed=0, rng_offset=0, row_offset=0, mean=None, want_mean_grad=True):
+    """Backward of `igso3_sample_exact` read as a reparameterised draw R = mean exp(angle hat(axis)), angle = F^{-1}(u; eps)
+    at fixed (u, axis).  angle (*shape) / axis (*shape,3): the forward's outputs; G (*shape,3,3): dL/dR.  eps / u / seed /
+    rng_offset / row_offset / mean as the forward got them (u and the Philox stream are read only at rows where eps == 0,
+    whose derivative is the eps -> 0+ limit 2 x0(u)).
+    -> (g_eps (*shape): dL/deps per row -- reduce it for a shared eps --, g_mean (*shape,3,3) = G N^T per row, or None)"""
+    shape = tuple(angle.shape)
+    dev = angle.device
+    n = angle.numel()
+    angle = check_f32(angle, "angle").contiguous()
+    axis = check_f32(axis, "axis", (3,)).expand(*shape, 3).contiguous()
+    G = check_f32(G, "G", (3, 3)).expand(*shape, 3, 3).contiguous()
+    eps_t, eps_stride = _per_row(eps, shape, dev, "eps")
+    if u is not None:
+        u = check_f32(u, "u").expand(shape).contiguous()
+    mean_stride = 0
+    if mean is not None:
+        mean = check_f32(mean, "mean", (3, 3))
+        if mean.numel() != 9:
+            mean = mean.expand(*shape, 3, 3).contiguous()
+            mean_stride = 1
+        else:
+            mean = mean.contiguous()
+    g_eps = torch.empty(shape, dtype=torch.float32, device=dev)
+    g_mean = torch.empty(*shape, 3, 3, dtype=torch.float32, device=dev) if want_mean_grad else None
+    call("so3d_igso3_rsample_bwd_f32", ptr(eps_t), eps_stride, ptr(angle), ptr(axis), ptr(mean), mean_stride, ptr(G), ptr(u),
+         int(seed), int(rng_offset), int(row_offset), ptr(g_eps), ptr(g_mean), n, device=dev)
+    return g_eps, g_mean
+
+
 # ---------------------------------------------------------------------------------------------
 # SE(3) arm: fused forward noising / reverse step on (rotation, translation) pairs (diffusion.py:432-573)
 # ---------------------------------------------------------------------------------------------
