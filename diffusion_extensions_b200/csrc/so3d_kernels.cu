@@ -1736,6 +1736,24 @@ struct RsampleBwdOp {
   }
 };
 
+// Entropy of IGSO(3)(eps) and its eps-derivative per row (IsotropicGaussianSO3.entropy; igso3_entropy, so3d_math.cuh): no
+// matrix or vector operands, 4 B in and 4 or 8 B out per row, so the engine stages nothing and each thread writes its scalars
+// directly.  The per-row cost depends on the regime (16 nodes of the image-free law, of the closed form, or of a 5-term
+// series), so rows run on the warp-autonomous schedule like the exact sampler.
+struct EntropyOp {
+  SO3D_OP_ARRAYS(0, 0, 0, 0)
+  SO3D_OP_NO_TAB
+  static constexpr bool kWarpSchedule = true;
+  const float* eps;
+  float* H;
+  float* dH;
+  __device__ void row(int64_t i, const Mat3*, const Vec3*, Mat3*, Vec3*, const float*) const {
+    float d;
+    H[i] = igso3_entropy(__ldg(eps + i), dH ? &d : nullptr);
+    if (dH) dH[i] = d;
+  }
+};
+
 // distributions.py:113-127 Bingham.rsample: unit quaternion = normalise(L z), z ~ N(0, I4), L = scale_tril of the
 // covariance; fused with util.py:222-252 quat_to_rmat (bingham_train.py:88-90 feeds the samples straight into it).
 struct BinghamOp {
@@ -3000,6 +3018,15 @@ int so3d_igso3_rsample_bwd_f32(const float* eps, int eps_stride, const float* an
   op.eps = eps; op.eps_stride = eps_stride; op.angle = angle; op.mean = mean; op.mean_stride = mean_stride;
   op.u_in = u; op.key = make_philox_key(seed, rng_offset); op.row_offset = row_offset; op.g_eps = g_eps;
   return launch_rowwise_pick(op, n, stream, "so3d_igso3_rsample_bwd_f32");
+}
+
+int so3d_igso3_entropy_f32(const float* eps, float* H, float* dH_deps, int64_t n, void* stream) {
+  SO3D_REQUIRE(n >= 0, "negative n");
+  if (n == 0) return 0;
+  SO3D_REQUIRE(eps && H, "so3d_igso3_entropy_f32: null pointer");
+  EntropyOp op;
+  op.eps = eps; op.H = H; op.dH = dH_deps;
+  return launch_rowwise_pick(op, n, stream, "so3d_igso3_entropy_f32");
 }
 
 int so3d_q_sample_f32(const float* x0, const int64_t* t, const float* sqrt_ac, const float* sqrt_1m_ac, int64_t T,

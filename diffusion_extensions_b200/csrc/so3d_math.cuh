@@ -1706,11 +1706,14 @@ SO3D_HD float igso3_angle_integrand(float x, float eps) {
   sincos_fast(eps * x, &s, &c);
   return x * s * expf(-x * x);
 }
+// 16-node Gauss-Legendre rule on [-1, 1]: the 8 positive nodes and their weights (shared with igso3_entropy)
+#define SO3D_GL16_NODES {9.501250984e-02f, 2.816035508e-01f, 4.580167777e-01f, 6.178762444e-01f, \
+                         7.554044084e-01f, 8.656312024e-01f, 9.445750231e-01f, 9.894009350e-01f}
+#define SO3D_GL16_WEIGHTS {1.894506105e-01f, 1.826034150e-01f, 1.691565194e-01f, 1.495959888e-01f, \
+                           1.246289713e-01f, 9.515851168e-02f, 6.225352394e-02f, 2.715245941e-02f}
 SO3D_HD AngleCdf igso3_angle_cdf_quad(float x, float eps, float C) {
-  constexpr float kNode[8] = {9.501250984e-02f, 2.816035508e-01f, 4.580167777e-01f, 6.178762444e-01f,
-                              7.554044084e-01f, 8.656312024e-01f, 9.445750231e-01f, 9.894009350e-01f};
-  constexpr float kWeight[8] = {1.894506105e-01f, 1.826034150e-01f, 1.691565194e-01f, 1.495959888e-01f,
-                                1.246289713e-01f, 9.515851168e-02f, 6.225352394e-02f, 2.715245941e-02f};
+  constexpr float kNode[8] = SO3D_GL16_NODES;
+  constexpr float kWeight[8] = SO3D_GL16_WEIGHTS;
   const float h = 0.5f * fminf(x, kExactXMax);
   float acc = 0.0f;
 #pragma unroll
@@ -1807,5 +1810,128 @@ SO3D_HD float igso3_angle_deps(float w, float eps) {
 // the Maxwell quantile, so dw/deps -> 2 x0(u).  x0 is the sampler's own quadrature-regime inversion at eps = 2^-64 (where
 // C sin(eps x) = (4/sqrt(pi)) x to fp32 and 2 eps x is exact): 2 x0 = 2^64 w.
 SO3D_HD float igso3_angle_deps_eps0(float u) { return igso3_angle_icdf(u, kTinyDown) * kTinyUp; }
+
+// ------------------------------------------------------------------------------------------------
+// Entropy of the IGSO(3) law and its eps-derivative (so3d_igso3_entropy_f32; DESIGN.md, "IGSO(3) entropy").  With f the
+// density w.r.t. normalised Haar measure, p(w) = f(w) (1 - cos w) / pi the angle law on [0, pi] and g = d log f / dw:
+//     H = -int_0^pi p log f dw,     dH/deps = 2 eps E_p[g^2]   (de Bruijn's identity on SO(3)).
+// The heat equation df/d(eps^2) = (sin^2(w/2) f')' / sin^2(w/2) (igso3_angle_deps) and one integration by parts give
+// dH/d(eps^2) = (2/pi) int sin^2(w/2) f'^2 / f = E_p[g^2]: the score the density evaluators already form, no second
+// derivative.  One pass over 16 Gauss-Legendre nodes gives both, with the sampler's switch at eps = 0.3:
+//   eps < kExactSeriesEps: the sampler's image-free law in x = w / (2 eps) on [0, kExactXMax].  There
+//        log f = (1/2) log pi + eps^2/4 - 3 log eps - x^2 - log sinc(eps x),   sinc t = sin t / t,
+//        and x has the density q = (4/sqrt(pi)) e^{eps^2/4} x^2 sinc(eps x) e^{-x^2} of mass 1, so
+//        H = 3 log eps - (1/2) log pi - eps^2/4 + E_q[x^2 + log sinc(eps x)],   dH/deps = (2/eps) E_q[(x - eps phi(w))^2]
+//        (g = phi(w) - x/eps).  Nothing inside a node scales with a power of eps: fp32 holds down to eps ~ 1e-38.
+//   kExactSeriesEps <= eps <= kAutoSeriesEps: the closed form (igso3_closed_f32, `auto`'s evaluator here), which keeps
+//        log f and g to full relative precision in the upper tail where f is ~1e-10; with E_haar over (1 - cos w)/pi on [0, pi]
+//        H = -E_haar[f log f],   dH/deps = 2 eps E_haar[f g^2].
+//        (The series delta-form below would lose every digit of 1 + delta there: its terms are 10^7 times the density.)
+//   eps > kAutoSeriesEps: f = 1 + delta, delta = sum_{l>=1} a_l chi_l(w) formed without the l = 0 term, and
+//        -H = E_haar[(1 + delta) log1p(delta) - delta],   dH/deps = 2 eps E_haar[delta'^2 / (1 + delta)].
+//        E_haar[delta] = 0, so the integrand is delta^2/2 + O(delta^3) and nothing cancels as -H -> (9/2) e^{-4 eps^2} (f - 1
+//        is ~1e-15 at eps = 3).  With chi_l = 1 + 2 sum_{m<=l} cos(m w) and the tails T_m = sum_{l>=m} a_l (per row, not
+//        per node):  delta = T_1 + 2 sum_m T_m cos(m w),  delta' = -2 sum_m m T_m sin(m w).
+// Quadrature error of the 16 nodes (fp64): <= 2.5e-9 absolute below eps = 0.3, <= 3.5e-10 relative above.  Special values:
+// the law depends on eps^2, so H is even and dH/deps odd in eps; eps = 0 gives H = -inf and dH/deps = +inf (the 0+ limit
+// 3/eps); NaN gives NaN; beyond kEntropyFlushEps (and from eps ~ 4.65 on, where (9/2) e^{-4 eps^2} < FLT_MIN) both are 0.
+constexpr int kEntropyTerms = 5;          // eps > 1: a_6 / a_1 = (13/3) e^{-40 eps^2} < 2e-17
+constexpr float kEntropyFlushEps = 8.0f;  // -H < (9/2) e^{-256}: 0 in fp32, and no inf * 0 at eps = inf
+
+// (1 + d) log1p(d) - d = d^2 (1/2 - d/6 + d^2/12 - ...), by its series for |d| < 1/8 (8 terms: <= 2e-9 relative)
+SO3D_HD float igso3_entropy_delta_term(float d) {
+  if (fabsf(d) < 0.125f) {
+    float s = fmaf(d, -1.3888889e-2f, 1.7857143e-2f);
+    s = fmaf(d, s, -2.3809524e-2f);
+    s = fmaf(d, s, 3.3333333e-2f);
+    s = fmaf(d, s, -5.0e-2f);
+    s = fmaf(d, s, 8.3333333e-2f);
+    s = fmaf(d, s, -1.6666667e-1f);
+    s = fmaf(d, s, 0.5f);
+    return d * d * s;
+  }
+  return fmaf(1.0f + d, log1pf(d), -d);
+}
+
+SO3D_HD float igso3_entropy(float eps, float* dH_deps) {
+  constexpr float kNode[8] = SO3D_GL16_NODES;
+  constexpr float kWeight[8] = SO3D_GL16_WEIGHTS;
+  const float e = fabsf(eps);
+  const float v = e * e;
+  float H, d;
+  if (isnan(e)) {
+    H = d = e;
+  } else if (e == 0.0f) {
+    H = -INFINITY;
+    d = INFINITY;
+  } else if (e < kExactSeriesEps) {
+    const float K = 2.2567583341910251f * expf(0.25f * v);  // 4 / sqrt(pi) e^{eps^2/4}
+    const float h = 0.5f * kExactXMax;
+    float sH = 0.0f, sG = 0.0f;
+#pragma unroll
+    for (int k = 0; k < 16; ++k) {
+      const float x = h * (k < 8 ? 1.0f - kNode[k] : 1.0f + kNode[k - 8]);
+      const float wq = h * kWeight[k < 8 ? k : k - 8];
+      const float t = e * x;
+      float s, c;
+      sincos_fast(t, &s, &c);
+      const float sinc = s / t;
+      const float q = wq * K * x * x * sinc * expf(-x * x);
+      const float r = fmaf(-e, igso3_angle_phi(2.0f * t), x);
+      sH = fmaf(q, fmaf(x, x, logf(sinc)), sH);
+      sG = fmaf(q, r * r, sG);
+    }
+    H = fmaf(3.0f, logf(e), fmaf(-0.25f, v, sH - 0.57236494292470008f));
+    d = (2.0f / e) * sG;
+  } else if (e <= kAutoSeriesEps) {
+    float sH = 0.0f, sG = 0.0f;
+#pragma unroll
+    for (int k = 0; k < 16; ++k) {
+      const float w = 0.5f * kPi * (k < 8 ? 1.0f - kNode[k] : 1.0f + kNode[k - 8]);
+      float sh, ch, lf, g;
+      sincos_fast(0.5f * w, &sh, &ch);
+      igso3_closed_f32(w, e, &lf, &g);
+      const float fq = kWeight[k < 8 ? k : k - 8] * sh * sh * expf(lf);
+      sH = fmaf(fq, lf, sH);
+      sG = fmaf(fq * g, g, sG);
+    }
+    H = -sH;
+    d = 2.0f * e * sG;
+  } else if (e < kEntropyFlushEps) {
+    float T[kEntropyTerms];
+    float tail = 0.0f;
+#pragma unroll
+    for (int l = kEntropyTerms; l >= 1; --l) {
+      tail = fmaf((float)(2 * l + 1), expf(-(float)(l * (l + 1)) * v), tail);
+      T[l - 1] = tail;
+    }
+    float sH = 0.0f, sG = 0.0f;
+#pragma unroll
+    for (int k = 0; k < 16; ++k) {
+      const float w = 0.5f * kPi * (k < 8 ? 1.0f - kNode[k] : 1.0f + kNode[k - 8]);
+      float sh, ch;
+      sincos_fast(0.5f * w, &sh, &ch);
+      const float s1 = 2.0f * sh * ch, c1 = fmaf(-2.0f * sh, sh, 1.0f);
+      float sm = s1, cm = c1, del = T[0], dp = 0.0f;
+#pragma unroll
+      for (int m = 1; m <= kEntropyTerms; ++m) {
+        del = fmaf(2.0f * T[m - 1], cm, del);
+        dp = fmaf(-2.0f * (float)m * T[m - 1], sm, dp);
+        const float sn = fmaf(sm, c1, cm * s1), cn = fmaf(cm, c1, -sm * s1);
+        sm = sn;
+        cm = cn;
+      }
+      const float hq = kWeight[k < 8 ? k : k - 8] * sh * sh;
+      sH = fmaf(hq, igso3_entropy_delta_term(del), sH);
+      sG = fmaf(hq * dp, dp / (1.0f + del), sG);
+    }
+    H = -sH;
+    d = 2.0f * e * sG;
+  } else {
+    H = d = 0.0f;
+  }
+  if (dH_deps) *dH_deps = eps < 0.0f ? -d : d;
+  return H;
+}
 
 }  // namespace so3d

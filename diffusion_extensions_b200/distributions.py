@@ -31,6 +31,9 @@ with ``reference_quirks=True`` raises.
 ``rsample`` is the reparameterised draw: always the exact inverse CDF (whatever ``sampler`` says), differentiable w.r.t. eps
 and the mean through one backward kernel.  At fixed (u, axis) the angle's derivative is dw/deps = -2 eps d log f / dw (the
 heat equation turns the implicit derivative -(dF/deps)/p into the angle score), evaluated at the sampled angle.
+``entropy`` is the entropy of the law w.r.t. normalised Haar measure (like ``rsample``, independent of the mean, ``mode``,
+``series_terms`` and ``sampler``), differentiable w.r.t. eps: the kernel also writes dH/deps = 2 eps E[(d log f / dw)^2]
+(de Bruijn's identity, the same heat equation), so the backward is one multiply.
 """
 import torch
 from torch.autograd.function import once_differentiable
@@ -79,6 +82,22 @@ class _RSample(torch.autograd.Function):
         if want_mean:
             g_mean = g_mean.reshape(-1, 9).sum(0).reshape(mean_shape) if mean.numel() == 9 else g_mean.sum_to_size(mean_shape)
         return g_eps, g_mean, None, None, None, None, None
+
+
+class _Entropy(torch.autograd.Function):
+    """H(eps), with dH/deps from the same launch saved for the backward."""
+
+    @staticmethod
+    def forward(ctx, eps):
+        H, dH = ops.igso3_entropy(eps, want_grad=ctx.needs_input_grad[0])
+        ctx.save_for_backward(dH)
+        return H
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad):
+        (dH,) = ctx.saved_tensors
+        return grad * dH
 
 
 class IsotropicGaussianSO3(Distribution):
@@ -170,6 +189,15 @@ class IsotropicGaussianSO3(Distribution):
         axes = None if axes is None else axes.detach()
         return _RSample.apply(self.eps, self._mean, eps_rows, shape, u, axes, row_offset)
 
+    def entropy(self):
+        """Entropy of IGSO(3)(eps) w.r.t. normalised Haar measure, shape eps.shape, differentiable w.r.t. eps (so KL(q || Haar)
+        = -entropy()).  The law's own entropy: independent of the mean, ``mode``, ``series_terms`` and ``sampler``.  Even in
+        eps; eps = 0 gives -inf with gradient +inf (the 0+ limit 3/eps).  Once differentiable."""
+        if self.reference_quirks:
+            raise ValueError("entropy is that of the IGSO(3) law itself; reference_quirks only shape the CDF table of "
+                             "sampler='table'")
+        return _Entropy.apply(self.eps)
+
     # -- density (distributions.py:53-72) --------------------------------------------------------
     def _eps_ft(self, t: torch.Tensor) -> torch.Tensor:
         t = t.to(device=self.eps.device, dtype=torch.float32)
@@ -222,7 +250,8 @@ class IsotropicGaussianSO3(Distribution):
 
 class IGSO3xR3(Distribution):
     """distributions.py:84-110: product of IGSO3(eps) on the rotation and N(shift, (eps * shift_scale)^2 I) on the
-    translation of an SE(3) element (`AffineT`).  `sample` draws both halves on the device; `rsample` too, differentiably."""
+    translation of an SE(3) element (`AffineT`).  `sample` draws both halves on the device; `rsample` too, differentiably.
+    `entropy` adds the two halves' entropies."""
 
     arg_constraints = {"eps": constraints.positive}
     has_rsample = True
@@ -251,6 +280,10 @@ class IGSO3xR3(Distribution):
         rot = self.igso3.rsample(sample_shape)
         shift = self.r3.rsample(sample_shape)
         return AffineT(rot, shift)
+
+    def entropy(self):
+        """Entropy of the product law: the IGSO(3) entropy plus that of the isotropic Gaussian shift, differentiable w.r.t. eps."""
+        return self.igso3.entropy() + self.r3.entropy().sum(-1)
 
     def log_prob(self, value):
         rot_prob = self.igso3.log_prob(value.rot)      # (..., 1)

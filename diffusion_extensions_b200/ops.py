@@ -500,6 +500,16 @@ def igso3_sample_exact(eps, shape, u=None, axes=None, seed=None, rng_offset=None
     return outs[0] if len(outs) == 1 else tuple(outs)
 
 
+def igso3_entropy(eps, want_grad=False):
+    """Entropy of IGSO(3)(eps) w.r.t. normalised Haar measure and its eps-derivative (de Bruijn: 2 eps E[(d log f / dw)^2]).
+    eps: float32 CUDA tensor of any shape.  -> (H, dH/deps or None), both shaped like eps."""
+    e = check_f32(eps, "eps")
+    H = torch.empty_like(e)
+    dH = torch.empty_like(e) if want_grad else None
+    call("so3d_igso3_entropy_f32", ptr(e), ptr(H), ptr(dH), e.numel(), device=e.device)
+    return H, dH
+
+
 def igso3_rsample_bwd(eps, angle, axis, G, u=None, seed=0, rng_offset=0, row_offset=0, mean=None, want_mean_grad=True):
     """Backward of `igso3_sample_exact` read as a reparameterised draw R = mean exp(angle hat(axis)), angle = F^{-1}(u; eps)
     at fixed (u, axis).  angle (*shape) / axis (*shape,3): the forward's outputs; G (*shape,3,3): dL/dR.  eps / u / seed /

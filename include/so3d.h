@@ -152,6 +152,15 @@ int so3d_igso3_rsample_bwd_f32(const float* eps, int eps_stride, const float* an
                                int mean_stride, const float* G9, const float* u, uint64_t seed, uint64_t rng_offset,
                                uint64_t row_offset, float* g_eps, float* g_mean9, int64_t n, void* stream);
 
+/* Entropy of IGSO(3)(eps) and its eps-derivative, per row (DESIGN.md 4.11):  H[i] = -int_0^pi p log f dw with
+ * p(w) = f(w) (1 - cos w) / pi, and dH_deps[i] = 2 eps E_p[(d log f / dw)^2] (de Bruijn's identity; dH_deps may be NULL:
+ * skipped).  One 16-node Gauss-Legendre pass: the image-free law in x = w / (2 eps) below eps = 0.3, the closed form up to
+ * eps = 1, the cancellation-free series form -H = E_haar[(1 + delta) log1p(delta) - delta], delta = f - 1, above.
+ * |error| <= 8 2^-24 (|H| + eps |dH/deps| + [eps <= 1]) for H and 8 2^-24 |dH/deps| (1 + 4 eps^2) for dH/deps, against
+ * fp64, for eps in [1e-20, 6] (results below FLT_MIN, from eps ~ 4.65 on, may flush to 0).  H is even and dH/deps odd in
+ * eps; eps = 0 gives -inf / +inf (the 0+ limit 3/eps), NaN gives NaN.  Runs on the persistent row engine. */
+int so3d_igso3_entropy_f32(const float* eps, float* H, float* dH_deps, int64_t n, void* stream);
+
 /* ---- L2: diffusion.py SO3Diffusion ---------------------------------------------------------- */
 /* diffusion.py:339-346 q_sample + :348-355 p_losses target, fused:
  *   eps = sqrt_1m_ac[t], noise ~ IGSO3(eps) from cdf row t, x_t = so3_scale(x0, sqrt_ac[t]) @ noise,
