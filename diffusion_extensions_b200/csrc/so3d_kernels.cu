@@ -947,6 +947,12 @@ __global__ void __launch_bounds__(kT2, OpMinCtas<Op>::value) rowwise_kernel_w2(c
       a3[a][1] = sm_vec(s_i3 + a * kRows2 * 3, r1);
     }
     if (kI9 + kI3 > 0) {
+      // kWarpIn: the refill below overwrites the slice these lanes have just read, through the async proxy.  Nothing but this
+      // __syncwarp stands between the two, so every lane orders its shared-memory reads before async-proxy writes (PTX: a
+      // generic-proxy access and a later async-proxy access to the same location need fence.proxy.async).  Without it the
+      // two-row forward-noising kernel at 2^24 rows now and then gave 16 rows of one warp a wrong x_t next to a right target
+      // and score: a wrong x0 read from the slice.
+      if (kWarpIn && tma && k + 1 < my_full) fence_proxy_async();
       __syncwarp();  // every lane's copy of its rows is complete
       if (kWarpIn) {
         if (tma && k + 1 < my_full && elect_one()) issue_warp_load(row0 + stride_rows);  // the next tile's slice loads behind the arithmetic

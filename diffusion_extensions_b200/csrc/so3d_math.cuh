@@ -1580,8 +1580,9 @@ SO3D_HD U4 philox4x32_10(const PhiloxRoundKeys& k, uint64_t row, uint64_t offset
   return c;
 }
 
-// 24-bit uniform in [0, 1), the same lattice torch.rand(float32) uses.  Device: one round-toward-zero conversion of the
-// whole word (keeps exactly the top 24 bits) and a multiply -- the same value as (x >> 8) 2^-24 without the shift.
+// Uniform in [0, 1) with 24 significant bits.  Device: one round-toward-zero conversion of the whole word (keeps its top 24
+// significant bits) and a multiply -- for x >= 2^31 the value (x >> 8) 2^-24 of the host branch (torch.rand's lattice),
+// finer below, where the word has leading zeros.
 SO3D_HD float u01(uint32_t x) {
 #if defined(__CUDA_ARCH__)
   return __uint2float_rz(x) * (1.0f / 4294967296.0f);

@@ -204,7 +204,7 @@ int so3d_p_sample_dseed_f32(const float* x_t, const float* pred3, const int64_t*
  * so3d_p_sample_f32 (shared t, rng_offset = rng_offset0 + t at step t), bit-identical to that sequence of launches.
  * Particles are independent, so a CTA keeps a chunk of them resident in shared memory for all steps: x_t is read from
  * HBM once and `out` written once (BASELINE configs[2]: 1000 steps x 2^24 particles).  post_cdf (T x 999) and its guide
- * records post_guide (T x 1024 x 4 words, so3d_igso3_cdf_guide) are required; out may alias x_t. */
+ * records post_guide (T x SO3D_GUIDE_BUCKETS x 4 words, so3d_igso3_cdf_guide) are required; out may alias x_t. */
 int so3d_p_sample_loop_f32(const float* x_t, const float* pred3, int64_t t_hi, int64_t t_lo, const float* recip, const float* recipm1,
                            const float* coef1, const float* coef2, int64_t T, const float* post_cdf, const uint32_t* post_guide,
                            const float* loc, uint64_t seed, uint64_t rng_offset0, uint64_t row_offset, float* out, int64_t n,

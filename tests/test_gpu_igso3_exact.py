@@ -3,10 +3,7 @@
 Accuracy with given u against the fp64 inverse CDF of the angle law (tests/igso3_angle_law.py), the law itself by a
 Kolmogorov-Smirnov test of the probability integral transform, the Philox draws it shares with the table sampler,
 the outputs and error cases, and the memory of a 2^24-row per-row-eps draw."""
-import ctypes
 import math
-import os
-import subprocess
 
 import numpy as np
 import pytest
@@ -15,10 +12,10 @@ from scipy import stats
 
 import diffusion_extensions_b200 as dx
 from diffusion_extensions_b200 import ops, util
+from tests import draws_ref as D
 from tests import igso3_angle_law as A
 
 pytestmark = pytest.mark.gpu
-HERE = os.path.dirname(os.path.abspath(__file__))
 PI32 = float(np.float32(math.pi))
 
 
@@ -101,26 +98,7 @@ def test_law_ks_and_isotropy(cuda_device, eps):
     assert np.abs(np.clip((tr - 1) / 2, -1, 1) - np.cos(w)).max() < 2e-6
 
 
-@pytest.fixture(scope="module")
-def philox(tmp_path_factory):
-    so = str(tmp_path_factory.mktemp("hm") / "host_math.so")
-    subprocess.check_call(["g++", "-O2", "-shared", "-fPIC", "-o", so, os.path.join(HERE, "host_math", "host_math.cpp")])
-    return ctypes.CDLL(so)
-
-
-def _device_u(philox, seed, row0, offset, n):
-    """The uniform the sampling kernels draw: word z of Philox(seed, row0 + i, offset), converted toward zero / 2^32."""
-    out = np.empty(4 * n, np.uint32)
-    philox.hm_philox(ctypes.c_ulonglong(seed), ctypes.c_ulonglong(row0), ctypes.c_ulonglong(offset),
-                     out.ctypes.data_as(ctypes.POINTER(ctypes.c_uint)), ctypes.c_long(n))
-    z = out.reshape(n, 4)[:, 2].astype(np.uint64)
-    bits = np.floor(np.log2(np.maximum(z, 1).astype(np.float64))).astype(np.int64) + 1
-    shift = np.maximum(bits - 24, 0).astype(np.uint64)
-    z = (z >> shift) << shift  # round toward zero to 24 significant bits
-    return (z.astype(np.float64) / 2.0 ** 32).astype(np.float32)
-
-
-def test_same_draws_as_the_table_sampler(cuda_device, philox):
+def test_same_draws_as_the_table_sampler(cuda_device):
     n, seed, off, row0 = 50_000, 0x1234_5678_9ABC, 3, 1000
     eps = torch.exp(torch.empty(n, device=cuda_device).uniform_(math.log(4.67e-3), 0.0))
     _, ang_x, ax_x = ops.igso3_sample_exact(eps, (n,), seed=seed, rng_offset=off, row_offset=row0, want_angle=True, want_axis=True)
@@ -129,8 +107,8 @@ def test_same_draws_as_the_table_sampler(cuda_device, philox):
     _, ang_t, ax_t = ops.igso3_sample(d.table, (n,), row_idx=row_idx, seed=seed, rng_offset=off, row_offset=row0, want_angle=True,
                                       want_axis=True)
     assert torch.equal(ax_x, ax_t)
-    # both samplers saw the u of the Philox layout: explicit u reproduces each one's angle bit for bit
-    u = torch.tensor(_device_u(philox, seed, row0, off, n), device=cuda_device)
+    # both samplers saw the u of the Philox layout (restated in numpy): explicit u reproduces each one's angle bit for bit
+    u = torch.tensor(D.u01(D.philox(seed, row0 + np.arange(n, dtype=np.uint64), off)[:, 2]), device=cuda_device)
     _, ang_xu = ops.igso3_sample_exact(eps, (n,), u=u, seed=seed, rng_offset=off, row_offset=row0, want_angle=True)
     _, ang_tu = ops.igso3_sample(d.table, (n,), row_idx=row_idx, u=u, seed=seed, rng_offset=off, row_offset=row0, want_angle=True)
     assert torch.equal(ang_xu, ang_x)
